@@ -18,6 +18,9 @@ first ONE pass over the whole survey, timed and hashed (`full_pass`), then W + K
 prepared + 31.5 S pairs matched each, the survey's own ratio) for the step-timed `value`.  Both arms print sha256
 digests of their inputs and of every output (per-pair counts, rows, keypoints, descriptors) in `config`: equal digests
 in the two arms and at every N = the whole workload is bit-identical.
+
+--dump-outputs DIR writes the outputs of the last timed step as .npy files (float32 / float64, at most 64 MB in all), so
+that two builds run with the same arguments, hence on the same seeded inputs, can be compared output for output.
 """
 import argparse
 import hashlib
@@ -38,8 +41,9 @@ if ROOT not in sys.path:
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of the resident leg and of each end-to-end leg (pipelined, isolated)")
+    ap.add_argument("--warmup", type=int, default=3, help="untimed resident steps before the timed ones (at least 3 are run; the "
+                    "end-to-end legs always warm up with 3 pipelined steps)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--images", type=int, default=64)
     ap.add_argument("--rows", type=int, default=8000)
@@ -59,7 +63,14 @@ def parse():
     ap.add_argument("--h2d-chunk", type=int, default=0, help="images per host-to-device chunk of the e2e pipeline (0 = library default)")
     ap.add_argument("--no-survey-call", action="store_true", help="e2e at N=1 through dsx_detect_feature_batch + dsx_match_pairs_dev instead of dsx_survey")
     ap.add_argument("--no-bruteforce", action="store_true", help="skip the match_cull=0 POPC-roofline leg and the frame_prepare leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="", help="after the timed steps, write what the last resident step "
+                    "computed (keypoints, descriptors, per-pair counts, correspondence rows) as DIR/<name>.npy; see dump_outputs")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
+    return a
 
 
 def workload_name(a):
@@ -86,6 +97,40 @@ def output_hashes(counts, rows6, kps_list, desc_list):
     """Digests of a survey's outputs (tests/test_gpu_ref.py::survey_hashes computes the same)."""
     return dict(counts=sha16(np.ascontiguousarray(counts, np.int32)), rows6=sha16(np.ascontiguousarray(rows6, np.float64)),
                 kps=sha16(*kps_list), desc=sha16(*desc_list))
+
+
+# bytes of each file of --dump-outputs (64 MB in all); an output above its share is written as a seeded sample of its rows
+DUMP_BYTES = dict(rows6=34 << 20, descriptors=16 << 20, keypoints=8 << 20, pair_counts=4 << 20, keypoint_counts=1 << 20)
+
+
+def dump_outputs(d, arrays):
+    """Writes every array of `arrays` (name -> float32 / float64 array, rows first) as d/<name>.npy.  An array larger
+    than DUMP_BYTES[name] is replaced by the rows a generator seeded with 0 picks (same row count -> same rows, so two
+    builds that agree on the counts are compared row for row); their row numbers go to d/<name>_rows.npy."""
+    os.makedirs(d, exist_ok=True)
+    for name, x in arrays.items():
+        assert x.dtype in (np.float32, np.float64), name
+        rows_path = os.path.join(d, name + "_rows.npy")
+        if x.nbytes > DUMP_BYTES[name]:
+            row_bytes = x.nbytes // len(x)
+            idx = np.sort(np.random.default_rng(0).choice(len(x), DUMP_BYTES[name] // (row_bytes + 8), replace=False))
+            x = x[idx]
+            np.save(rows_path, idx.astype(np.float64))
+        elif os.path.exists(rows_path):
+            os.remove(rows_path)
+        np.save(os.path.join(d, name + ".npy"), np.ascontiguousarray(x))
+
+
+def step_outputs(cnt_pairs, rows6, kps_list, desc_list):
+    """What a caller of the survey path receives, as float arrays: per-pair row counts (in the order of the step's pair
+    list), the correspondence rows, and the keypoints (cv::KeyPoint fields x, y, size, angle, response, octave, class_id) and
+    descriptor bytes of every image, concatenated in image order, with the keypoint count of every image."""
+    from diasss_b200.binding import KP_DTYPE
+    kp = np.ascontiguousarray(np.concatenate(kps_list) if kps_list else np.zeros((0, 7), np.float32)).view(KP_DTYPE).reshape(-1)
+    return dict(pair_counts=np.asarray(cnt_pairs, np.float64), rows6=np.asarray(rows6, np.float64),
+                keypoints=np.stack([kp[f].astype(np.float64) for f in KP_DTYPE.names], 1),
+                descriptors=(np.concatenate(desc_list) if desc_list else np.zeros((0, 32), np.uint8)).astype(np.float32),
+                keypoint_counts=np.array([len(k) for k in kps_list], np.float64))
 
 
 def make_config(a, inputs_sha, kp_total, n_corr, hashes, cand0, n_pairs=None):
@@ -581,6 +626,8 @@ def run_ours(a):
         kps_l = [feats_all["kps"][int(sl), :int(kc[int(sl)])].cpu().numpy() for sl in slot_of_image]
         desc_l = [feats_all["desc"][int(sl), :int(kc[int(sl)])].cpu().numpy() for sl in slot_of_image]
         hashes = output_hashes(cnt_pairs, rows_np, kps_l, desc_l)
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, step_outputs(cnt_pairs, rows_np, kps_l, desc_l))
         del kps_l, desc_l, rows_np
         # FAST candidates per level of image 0 (the density the FAST / quadtree stages see)
         one = fe.alloc_features(1)
@@ -768,7 +815,7 @@ def run_ours(a):
         run_pipelined(3)
         ms_e2e = timed_e2e(run_pipelined, a.steps)
         e2e_rows_sha = sha16(h_rows[:int(h_tot[(a.steps - 1) & 1])].numpy()) if rank == 0 else None
-        ms_iso = timed_e2e(run_isolated, max(2, min(a.steps, 6)))
+        ms_iso = timed_e2e(run_isolated, a.steps)
         fe.ctx.check_error()
         d2h = state["d2h"]
         # images and the geo model are copied; of the masks only the 32-byte sectors under the <= cap keypoints per image

@@ -8,6 +8,8 @@ restatement.  The libraries are prebuilt artefacts that travel to the GPU box; /
   config 3   the 16-image / 120-pair survey: sha256 over counts, rows, keypoints and descriptors of the WHOLE workload
              (src/diasss2.cpp:82-97 on the reference's classes, over host threads) == the device path's
   libm       the device's cosf / sinf against the host libm the reference links
+  config 4   bench.py's 64-frame survey against the digests the reference build produced on it (stored under
+             tests/golden, so this one runs without oracle/_ref)
 """
 import ctypes
 import hashlib
@@ -24,7 +26,7 @@ pytestmark = pytest.mark.gpu
 def ref(built):
     from oracle import ref as R
     if not R.available():
-        pytest.skip("oracle/_ref is not built")
+        pytest.skip("oracle/_ref is not built: oracle/build_ref.sh needs the reference's sources (DSX_REFERENCE_ROOT)")
     for strict in (False, True):
         R.set_modes(heap_monotone=True, libm_a5=False, mean_order=1, strict=strict)
     return R
@@ -138,6 +140,35 @@ def test_config3_whole_survey_hashes_vs_reference_build(oracle, ref):
         assert ov.tobytes() == out["overlap"].tobytes()
     finally:
         fe.ctx.close()
+
+
+def test_bench_survey_vs_recorded_reference_digests(built, tmp_path):
+    """BASELINE config 4 where no reference build is at hand: bench.py's survey (64 frames of 8000 x 2000, 2016 pairs)
+    through the device path has the inputs, FAST candidate counts and output digests that the reference's own sources
+    produced on it (tests/golden/reference_survey.json, recorded by `bench.py --impl reference`).  The step's
+    --dump-outputs arrays hash to the same digests, so they are exactly what the step computed."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    want = json.load(open(os.path.join(root, "tests", "golden", "reference_survey.json")))["config"]
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "1", "--warmup", "0", "--no-e2e", "--no-cpu-baseline",
+                        "--no-bruteforce", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=1800)
+    assert r.returncode == 0, r.stderr[-3000:]
+    got = json.loads(r.stdout.strip().splitlines()[-1])["config"]
+    for k, v in want.items():
+        assert got[k] == v, k
+    out = {n: np.load(tmp_path / (n + ".npy")) for n in ("pair_counts", "keypoint_counts", "keypoints", "descriptors", "rows6")}
+    from diasss_b200.binding import KP_DTYPE
+    kp = np.zeros(len(out["keypoints"]), KP_DTYPE)
+    for i, f in enumerate(KP_DTYPE.names):
+        kp[f] = out["keypoints"][:, i]
+    sha = lambda x: hashlib.sha256(np.ascontiguousarray(x).tobytes()).hexdigest()[:16]
+    assert sha(out["pair_counts"].astype(np.int32)) == want["output_sha256"]["counts"]
+    assert sha(kp) == want["output_sha256"]["kps"] and sha(out["descriptors"].astype(np.uint8)) == want["output_sha256"]["desc"]
+    assert out["pair_counts"].sum() == want["correspondences"] and out["keypoint_counts"].sum() == len(kp)
+    assert len(out["rows6"]) > 0 and sum(p.stat().st_size for p in tmp_path.iterdir()) <= 64 << 20
 
 
 def test_device_sincosf_is_the_host_libm(frontend):

@@ -24,7 +24,7 @@ from tests._util import oracle_frame, textured
 def ref(built):
     from oracle import ref as R
     if not R.available():
-        pytest.skip("oracle/_ref is not built and /root/reference is absent")
+        pytest.skip("oracle/_ref is not built: oracle/build_ref.sh needs the reference's sources (DSX_REFERENCE_ROOT)")
     R.set_modes(heap_monotone=True, libm_a5=False, mean_order=0)
     R.set_modes(heap_monotone=True, libm_a5=False, mean_order=0, strict=True)
     return R
