@@ -52,6 +52,7 @@ EXPORTS = [
     "dsx_features_free", "dsx_detect_feature_batch_dev", "dsx_detect_feature_batch", "dsx_geo_model_build", "dsx_geo_model_build_batch", "dsx_georef_batch_dev",
     "dsx_match_pairs_dev", "dsx_survey", "dsx_frame_prepare_batch_dev", "dsx_compute_intersection", "dsx_build_pair_list", "dsx_check_error", "dsx_launch_count", "dsx_timing_enable", "dsx_timing_read", "dsx_stage_name", "dsx_popc_peak",
     "dsx_peer_create", "dsx_peer_connect", "dsx_peer_connect_local", "dsx_match_pairs_peer", "dsx_peer_collect", "dsx_peer_destroy",
+    "dsx_group_create", "dsx_group_destroy", "dsx_group_ctx", "dsx_group_blocks", "dsx_group_survey_host",
     "dsx_io_read_matrix", "dsx_io_write_matrix", "dsx_io_read_column",
     "dsx_debug_level_image", "dsx_debug_candidates", "dsx_debug_level_keys", "dsx_debug_match", "dsx_debug_sincosf", "dsx_debug_fast_profile", "dsx_survey_host", "dsx_get_kps_pairs_dev",
 ]
@@ -75,6 +76,8 @@ def lib():
         L.dsx_features_free.restype = None
         L.dsx_default_params.restype = None
         L.dsx_peer_destroy.restype = None
+        L.dsx_group_destroy.restype = None
+        L.dsx_group_ctx.restype = C.c_void_p
         _lib = L
     return _lib
 
@@ -371,6 +374,76 @@ class Peer:
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
             lib().dsx_peer_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class _GroupContext(Context):
+    """A context owned by a Group (dsx_group_ctx): usable like a Context, destroyed with the group."""
+
+    def __init__(self, handle, params):
+        self.params = params
+        self._h = C.c_void_p(handle)
+        self.cap = int(lib().dsx_max_keypoints(self._h))
+        self.nlevels = params.nlevels
+
+    def close(self):
+        self._h = C.c_void_p()
+
+
+def group_blocks(n_images, n_devices, image_counts=None):
+    """dsx_group_blocks: first frame of every device's block (n_devices + 1 entries, last = n_images)."""
+    first = np.empty(n_devices + 1, np.int32)
+    counts = None if image_counts is None else np.ascontiguousarray(image_counts, np.int32)
+    if counts is not None and len(counts) != n_devices:
+        raise DsxError(ERR_INVALID, "image_counts needs one entry per device")
+    _chk(lib().dsx_group_blocks(int(n_images), int(n_devices), _p(counts), _p(first)))
+    return first
+
+
+class Group:
+    """dsx_group: one process driving several GPUs (a device may be listed more than once); see include/diasss_b200.h."""
+
+    def __init__(self, devices, **params):
+        self.devices = [int(d) for d in devices]
+        self.params = default_params(**params)
+        self._h = C.c_void_p()
+        devs = np.ascontiguousarray(self.devices, np.int32) if self.devices else None
+        _chk(lib().dsx_group_create(C.byref(self.params), _p(devs), len(self.devices), C.byref(self._h)))
+        self.ctxs = [_GroupContext(lib().dsx_group_ctx(self._h, i), self.params) for i in range(len(self.devices))]
+        self.cap = self.ctxs[0].cap
+
+    def survey_host(self, images_ptr, masks_ptr, n_images, rows, cols, step, img_stride, poses, g_ranges, img_id, pairs, feats,
+                    corr_count_ptr, corr_offset_ptr, rows6_ptr, cap_rows, image_counts=None, sync=True, bbox_out=None):
+        """dsx_group_survey_host: Context.survey_host on every device of the group, outputs on devices[0]."""
+        img_id = np.ascontiguousarray(img_id, np.int32)
+        pairs = np.ascontiguousarray(pairs, np.int32).reshape(-1, 2)
+        counts = None if image_counts is None else np.ascontiguousarray(image_counts, np.int32)
+        if counts is not None and len(counts) != len(self.devices):
+            raise DsxError(ERR_INVALID, "image_counts needs one entry per device")
+        assert poses.dtype == np.float64 and poses.flags.c_contiguous and g_ranges.dtype == np.float64 and g_ranges.flags.c_contiguous
+        kt = C.c_int64()
+        _chk(lib().dsx_group_survey_host(self._h, _p(images_ptr), _p(masks_ptr) if masks_ptr else C.c_void_p(0), n_images, rows, cols,
+                                         C.c_size_t(step), C.c_size_t(img_stride), _p(poses), _p(g_ranges), g_ranges.shape[1], _p(img_id),
+                                         _p(pairs), len(pairs), _p(counts), C.byref(feats), _p(corr_count_ptr), _p(corr_offset_ptr),
+                                         _p(rows6_ptr), C.c_int64(cap_rows), C.byref(kt) if sync else C.c_void_p(0),
+                                         _p(bbox_out) if bbox_out is not None else C.c_void_p(0)))
+        return kt.value if sync else None
+
+    def check_error(self):
+        for c in self.ctxs:
+            c.check_error()
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h.value:
+            for c in self.ctxs:
+                c.close()
+            lib().dsx_group_destroy(self._h)
             self._h = C.c_void_p()
 
     def __del__(self):

@@ -15,7 +15,7 @@
 namespace dsx {
 
 static thread_local std::string t_error;
-int64_t g_launches = 0;
+std::atomic<int64_t> g_launches{0};
 void set_error(const std::string& s) { t_error = s; }
 void init_tables(dsx_ctx* ctx);
 int upload_umax(dsx_ctx* ctx);
@@ -336,7 +336,7 @@ void dsx_default_params(dsx_params* p) {
 
 const char* dsx_last_error(void) { return t_error.c_str(); }
 const char* dsx_version(void) { return "diasss_b200 0.1 (sm_100a)"; }
-int64_t dsx_launch_count(void) { return g_launches; }
+int64_t dsx_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
 
 int dsx_create(const dsx_params* params, void* stream, dsx_ctx** out) {
     if (!out) { set_error("null out"); return DSX_ERR_INVALID; }

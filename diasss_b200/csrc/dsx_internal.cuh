@@ -5,6 +5,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <atomic>
+
 #include <string>
 #include <vector>
 
@@ -21,7 +23,7 @@ constexpr int kMaxDim = 32760;    // coordinates are packed in 16 bits
 constexpr unsigned long long kBestOrderMask = 0x00ffffffffffffffull;
 
 void set_error(const std::string& s);
-extern int64_t g_launches;
+extern std::atomic<int64_t> g_launches;   // kernels launched (several host threads launch at once)
 
 #define DSX_CUDA(expr)                                                                             \
     do {                                                                                           \
@@ -40,7 +42,7 @@ extern int64_t g_launches;
 
 #define DSX_LAUNCH_CHECK()                                                            \
     do {                                                                              \
-        dsx::g_launches++;                                                            \
+        dsx::g_launches.fetch_add(1, std::memory_order_relaxed);                     \
         cudaError_t _e = cudaGetLastError();                                          \
         if (_e != cudaSuccess) {                                                      \
             dsx::set_error(std::string("kernel launch: ") + cudaGetErrorString(_e)); \
@@ -296,7 +298,7 @@ struct StageTimer {
         else cudaEventCreate(&e);
         return e;
     }
-    StageTimer(dsx_ctx* c, int s) : ctx(c), stage(s), l0(g_launches) {
+    StageTimer(dsx_ctx* c, int s) : ctx(c), stage(s), l0(g_launches.load(std::memory_order_relaxed)) {
         if (!ctx->timing) return;
         a = get(ctx); b = get(ctx);
         cudaEventRecord(a, ctx->stream);
@@ -305,7 +307,7 @@ struct StageTimer {
         if (!ctx->timing) return;
         cudaEventRecord(b, ctx->stream);
         ctx->spans.push_back({stage, a, b});
-        ctx->stage_launches[stage] += g_launches - l0;
+        ctx->stage_launches[stage] += g_launches.load(std::memory_order_relaxed) - l0;
     }
 };
 

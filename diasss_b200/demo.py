@@ -18,6 +18,7 @@ write_survey() stores frames in the same formats (the test-suite's stand-in for 
 Host I/O only moves bytes; everything numeric runs in libdiasss_b200.so.
 
 CLI:  python -m diasss_b200.demo --image DIR --pose DIR --altitude DIR --groundrange DIR [--annotation DIR] [--out F.npz]
+          [--gpus N]     (N > 1: extraction and matching on devices 0..N-1 of this process, dsx_group_survey_host; same output)
 """
 import argparse
 import os
@@ -63,9 +64,10 @@ def write_survey(root, raws, poses, altitudes, granges, annos=None, first_id=170
     return {k: os.path.join(root, v) for k, v in names.items()}
 
 
-def front_end(data, device=0, min_overlap=MIN_OVERLAP, **params):
+def front_end(data, device=0, min_overlap=MIN_OVERLAP, gpus=1, **params):
     """Frames + correspondences of a loaded survey (all images of one shape).  Returns dict(frames=[dict(img_id, kps,
-    desc, norm_img, flt_mask, bbox, corres_kps)], pairs, overlap, count, rows6)."""
+    desc, norm_img, flt_mask, bbox, corres_kps)], pairs, overlap, count, rows6).  gpus > 1: DetectFeature and the matching
+    run on devices 0..gpus-1 (one dsx_group_survey_host call on the host frames); the frames are prepared on `device`."""
     import torch
     from .frontend import FrontEnd
     raws = data["imgs"]
@@ -87,12 +89,25 @@ def front_end(data, device=0, min_overlap=MIN_OVERLAP, **params):
         tabs, bboxes = B.geo_model_build_batch(np.stack(data["poses"]), rows, cols, gr)     # host threads, same libm calls as the reference
         rowtabs = torch.from_numpy(tabs).to(dev)
         granges = torch.from_numpy(gr).to(dev)
-        feats = fe.alloc_features(n)
-        fe.ctx.detect_feature_batch_dev(norm.data_ptr(), mask.data_ptr(), n, rows, cols, step, rows * step, feats["c"])
-        fe.ctx.georef_batch_dev(feats["c"], rowtabs.data_ptr(), granges.data_ptr(), rows, cols, n_range)
         pairs, overlap = B.build_pair_list(bboxes, min_overlap)
         ids = list(range(n))                                     # Frame(i, ...): img_id = position in the sorted list
-        res = fe.match_pairs(feats, ids, [rows] * n, bboxes, pairs) if len(pairs) else None
+        if gpus > 1:
+            from .frontend import SurveyGroup
+            sg = SurveyGroup(list(range(gpus)), **params)
+            try:
+                h_norm = torch.from_numpy(np.ascontiguousarray(norm.cpu().numpy()[:, :, :cols])).pin_memory()
+                h_mask = torch.from_numpy(np.ascontiguousarray(mask.cpu().numpy()[:, :, :cols])).pin_memory()
+                res = sg.process_survey_host(h_norm, h_mask, np.stack(data["poses"]), gr, ids, pairs)
+                feats = res["feats"]
+                if not len(pairs):
+                    res = None
+            finally:
+                sg.close()
+        else:
+            feats = fe.alloc_features(n)
+            fe.ctx.detect_feature_batch_dev(norm.data_ptr(), mask.data_ptr(), n, rows, cols, step, rows * step, feats["c"])
+            fe.ctx.georef_batch_dev(feats["c"], rowtabs.data_ptr(), granges.data_ptr(), rows, cols, n_range)
+            res = fe.match_pairs(feats, ids, [rows] * n, bboxes, pairs) if len(pairs) else None
         cnt = res["count"].cpu().numpy()[:len(pairs)] if res else np.zeros(0, np.int32)
         rows6 = res["rows6"].cpu().numpy() if res else np.zeros((0, 6))
         nk = feats["count"].cpu().numpy()
@@ -121,11 +136,12 @@ def main(argv=None):
     ap.add_argument("--annotation", default=None)
     ap.add_argument("--out", default=None, help="write keypoints / descriptors / corres_kps of every frame to this .npz")
     ap.add_argument("--device", type=int, default=0)
+    ap.add_argument("--gpus", type=int, default=1, help="extract and match on devices 0..N-1 of this process (same output)")
     a = ap.parse_args(argv)
     data = load_input_data(a.image, a.pose, a.altitude, a.groundrange, a.annotation)
     for k, im in enumerate(data["imgs"]):
         print("image size: %d %d" % im.shape)                   # (util.cpp:94)
-    res = front_end(data, device=a.device)
+    res = front_end(data, device=a.device, gpus=a.gpus)
     q = 0
     n = len(res["frames"])
     for i in range(n):

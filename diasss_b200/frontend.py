@@ -9,6 +9,8 @@ Reference interface                                        ->  here
   FEAmatcher::GeoNearNeighSearch(...)                      ->  FrontEnd.geo_near_neigh_search   :52-321
   FEAmatcher::DescriptorDistance(a, b)                     ->  FrontEnd.descriptor_distance     :442-458
   test_demo's two loops (diasss2.cpp:82-97)                ->  FrontEnd.process_survey (device-resident, batched)
+                                                               FrontEnd.process_survey_host (host images and poses in)
+                                                               SurveyGroup.process_survey_host (the same on several GPUs)
 
 The C++ twin of this file is include/diasss_b200/shim.hpp.  Everything numeric happens in libdiasss_b200.so (CUDA);
 this module only moves buffers.  torch is used for device memory and streams in the batched path.
@@ -119,6 +121,18 @@ class FrontEnd:
         self.ctx.georef_batch_dev(feats["c"], rowtabs.data_ptr(), g_ranges.data_ptr(), rows, cols, g_ranges.shape[1])
         return self.match_pairs(feats, img_ids, [rows] * F_, bboxes, pairs, out=out)
 
+    def process_survey_host(self, images, masks, poses, g_ranges, img_ids, pairs, feats=None, out=None, sync=True):
+        """test_demo's two hot loops from host data (dsx_survey_host): the per-ping geo model is built inside.
+
+        images, masks : uint8 host arrays [F, rows, cols] (torch CPU tensors, pinned or not, or numpy arrays; masks may be None)
+        poses         : float64 host [F, rows, 6];  g_ranges: float64 host [F, n_range]
+        img_ids       : host [F];  pairs: host int32 [P,2] indices into the F images
+        Returns dict(feats, count[P], offset[P+1], rows6[K,6], k, bbox[F,4]) -- device tensors on this GPU; K and bbox on the host.
+        sync=False: nothing is read back (k is None, rows6 is the whole output buffer).
+        """
+        return _survey_host(self, lambda *a, **kw: self.ctx.survey_host(*a, **kw), images, masks, poses, g_ranges, img_ids, pairs,
+                            feats, out, sync)
+
     def alloc_features(self, n_images):
         """Feature block as torch tensors (so it can be all-gathered with torch.distributed) + its C descriptor."""
         import torch
@@ -162,3 +176,62 @@ class FrontEnd:
         return dict(count=torch.zeros(max(n_pairs, 1), dtype=torch.int32, device=dev),
                     offset=torch.zeros(n_pairs + 1, dtype=torch.int32, device=dev),
                     rows6=torch.zeros(max(n_pairs, 1) * rows_per_pair, 6, dtype=torch.float64, device=dev))
+
+
+def _host_ptr(a):
+    if a is None:
+        return 0
+    if isinstance(a, np.ndarray):
+        assert a.dtype == np.uint8 and a.flags.c_contiguous
+        return a.ctypes.data
+    assert not a.is_cuda and a.is_contiguous() and a.dtype.itemsize == 1
+    return a.data_ptr()
+
+
+def _survey_host(fe, call, images, masks, poses, g_ranges, img_ids, pairs, feats, out, sync, **kw):
+    F_, rows, cols = images.shape
+    poses = np.ascontiguousarray(poses, np.float64).reshape(F_, rows, 6)
+    g_ranges = np.ascontiguousarray(g_ranges, np.float64).reshape(F_, -1)
+    pairs = np.ascontiguousarray(pairs, np.int32).reshape(-1, 2)
+    if feats is None:
+        feats = fe.alloc_features(F_)
+    if out is None:
+        out = fe.alloc_match_out(len(pairs), feats["count"].device)
+    bbox = np.zeros((F_, 4), np.float64)
+    k = call(_host_ptr(images), _host_ptr(masks), F_, rows, cols, cols, rows * cols, poses, g_ranges, img_ids, pairs, feats["c"],
+             out["count"].data_ptr(), out["offset"].data_ptr(), out["rows6"].data_ptr(), out["rows6"].shape[0], sync=sync,
+             bbox_out=bbox, **kw)
+    return dict(feats=feats, count=out["count"], offset=out["offset"], rows6=out["rows6"][:k] if sync else out["rows6"], k=k,
+                bbox=bbox)
+
+
+class SurveyGroup(FrontEnd):
+    """The diasss front end on several GPUs of one process (dsx_group): devices[i] is a CUDA ordinal, and one may be
+    listed more than once (logical ranks on one GPU).  Outputs land on devices[0], byte for byte what FrontEnd on one GPU
+    produces.  The single-GPU entry points of FrontEnd run on devices[0]."""
+
+    def __init__(self, devices, **params):
+        params.pop("device", None)
+        self.group = B.Group(devices, **params)
+        self.devices = self.group.devices
+        self.ctx = self.group.ctxs[0]
+        self.orb = ORBextractor(_ctx=self.ctx)
+
+    def process_survey_host(self, images, masks, poses, g_ranges, img_ids, pairs, feats=None, out=None, sync=True, image_counts=None):
+        """FrontEnd.process_survey_host on the group's GPUs.  image_counts: frames per device (contiguous blocks in image
+        order; None = as equal as possible)."""
+        import torch
+        with torch.cuda.device(self.devices[0]):
+            return _survey_host(self, self.group.survey_host, images, masks, poses, g_ranges, img_ids, pairs, feats, out, sync,
+                                image_counts=image_counts)
+
+    def alloc_features(self, n_images):
+        import torch
+        with torch.cuda.device(self.devices[0]):
+            return super().alloc_features(n_images)
+
+    def check_error(self):
+        self.group.check_error()
+
+    def close(self):
+        self.group.close()

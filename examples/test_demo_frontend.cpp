@@ -1,10 +1,12 @@
 // test_demo's front end (src/diasss2.cpp:26-97, everything before Optimizer::TrajOptimizationAll) on a B200, written
 // against the C ABI only -- no OpenCV, no Boost, no GTSAM.  It takes the reference's own command line
-//     test_demo_frontend --image DIR --pose DIR --altitude DIR --groundrange DIR [--annotation DIR] [--out FILE]
+//     test_demo_frontend --image DIR --pose DIR --altitude DIR --groundrange DIR [--annotation DIR] [--out FILE] [--gpus N]
 // loads the folders the way Util::LoadInputData does (files in name order; FileStorage XML nodes ct_img / auv_pose,
 // one-number-per-line text files), builds the frames on the device (GetNormalizeSSS, GetFilteredMask, geo model,
 // DetectFeature), runs the overlap-gated i<j loop with FEAmatcher::RobustMatching and prints the reference's
 // "OVERLAPPING RATE" lines.  --out writes every matched pair's corres_kps rows [id_s id_t y_s x_s y_t x_t] as text.
+// --gpus N (default 1) extracts and matches on devices 0..N-1 of this process with one dsx_group_survey_host call (host
+// images and poses in); the output is the same.
 //
 // Build (see __graft_entry__.build()):
 //   g++ -std=c++11 -O2 examples/test_demo_frontend.cpp -Iinclude -I/usr/local/cuda/include -Ldiasss_b200 -ldiasss_b200
@@ -50,13 +52,15 @@ static std::vector<std::string> sorted_files(const std::string& dir) {      // u
 int main(int argc, char** argv) {
     const float MIN_OVERLAP = 0.4f;                                          // diasss2.cpp:28
     std::string image, pose, altitude, groundrange, annotation, out_path;
+    int gpus = 1;
     for (int i = 1; i + 1 < argc; i += 2) {
         const std::string k = argv[i];
+        if (k == "--gpus") { gpus = std::max(1, atoi(argv[i + 1])); continue; }
         (k == "--image" ? image : k == "--pose" ? pose : k == "--altitude" ? altitude : k == "--groundrange" ? groundrange :
          k == "--annotation" ? annotation : out_path) = argv[i + 1];
     }
     if (image.empty() || pose.empty() || altitude.empty() || groundrange.empty()) {
-        printf("usage: %s --image DIR --pose DIR --altitude DIR --groundrange DIR [--annotation DIR] [--out FILE]\n", argv[0]);
+        printf("usage: %s --image DIR --pose DIR --altitude DIR --groundrange DIR [--annotation DIR] [--out FILE] [--gpus N]\n", argv[0]);
         return 0;
     }
     // --- parse input data (Util::LoadInputData)
@@ -108,8 +112,10 @@ int main(int argc, char** argv) {
     CU(cudaMemcpy(d_gr, gr_packed.data(), gr_packed.size() * 8, cudaMemcpyHostToDevice));
     dsx_features_dev feats;
     CK(dsx_features_alloc(ctx, F, &feats));
-    CK(dsx_detect_feature_batch_dev(ctx, d_norm, d_mask, F, rows, cols, step, step * rows, &feats));
-    CK(dsx_georef_batch_dev(ctx, &feats, d_rowtab, d_gr, rows, cols, n_range));
+    if (gpus == 1) {
+        CK(dsx_detect_feature_batch_dev(ctx, d_norm, d_mask, F, rows, cols, step, step * rows, &feats));
+        CK(dsx_georef_batch_dev(ctx, &feats, d_rowtab, d_gr, rows, cols, n_range));
+    }
     // --- find correspondences between each pair of frames (diasss2.cpp:88-97)
     const int all_pairs = F * (F - 1) / 2;
     std::vector<int32_t> pairs(2 * (size_t)std::max(all_pairs, 1));
@@ -128,7 +134,22 @@ int main(int argc, char** argv) {
     CU(cudaMalloc((void**)&d_off, sizeof(int32_t) * (n_pairs + 1)));
     CU(cudaMalloc((void**)&d_rows6, sizeof(double) * 6 * cap_rows));
     int64_t k_total = 0;
-    if (n_pairs > 0)
+    dsx_group* group = nullptr;
+    uint8_t *h_norm = nullptr, *h_mask = nullptr;
+    if (gpus > 1) {
+        // the same two loops on devices 0..gpus-1: frames in contiguous blocks per device, features exchanged over peer
+        // copies, the pair list cut into blocks, rows collected in pair order on device 0 (where feats and d_rows6 live)
+        std::vector<int> devices(gpus);
+        for (int d = 0; d < gpus; d++) devices[d] = d;
+        CK(dsx_group_create(nullptr, devices.data(), gpus, &group));
+        CU(cudaMallocHost((void**)&h_norm, step * rows * F));
+        CU(cudaMallocHost((void**)&h_mask, step * rows * F));
+        CU(cudaMemcpy(h_norm, d_norm, step * rows * F, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(h_mask, d_mask, step * rows * F, cudaMemcpyDeviceToHost));
+        CK(dsx_group_survey_host(group, h_norm, h_mask, F, rows, cols, step, step * rows, poses.data(), gr_packed.data(), n_range,
+                                 img_id.data(), pairs.data(), n_pairs, nullptr, &feats, d_cnt, d_off, d_rows6, cap_rows, &k_total,
+                                 nullptr));
+    } else if (n_pairs > 0)
         CK(dsx_match_pairs_dev(ctx, &feats, img_id.data(), img_rows.data(), bbox.data(), pairs.data(), n_pairs, d_cnt, d_off, d_rows6,
                                cap_rows, &k_total));
     std::vector<double> rows6(6 * (size_t)std::max<int64_t>(k_total, 1));
@@ -152,6 +173,7 @@ int main(int argc, char** argv) {
     }
     dsx_features_free(&feats);
     cudaFree(d_raw); cudaFree(d_norm); cudaFree(d_mask); cudaFree(d_rowtab); cudaFree(d_gr); cudaFree(d_cnt); cudaFree(d_off); cudaFree(d_rows6);
+    if (group) { dsx_group_destroy(group); cudaFreeHost(h_norm); cudaFreeHost(h_mask); }
     dsx_destroy(ctx);
     return 0;
 }

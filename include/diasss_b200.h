@@ -317,6 +317,38 @@ int dsx_peer_collect(dsx_ctx* ctx, dsx_peer* peer, int seq, const int32_t** corr
 void dsx_peer_destroy(dsx_peer* peer);
 
 /* ------------------------------------------------------------------------------------------------
+ * Several GPUs from one process (SURVEY.md section 5: single process, n devices, plain peer copies; no MPI, NCCL or IPC
+ * handles).  A group holds one dsx_ctx per entry of devices[], each with its own stream and host worker thread.  A device
+ * may be listed more than once (logical ranks on one GPU, as dsx_peer_connect_local allows).
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct dsx_group dsx_group;
+int dsx_group_create(const dsx_params* params, const int* devices, int n_devices, dsx_group** out);
+void dsx_group_destroy(dsx_group* g);
+/* Context of devices[i] (NULL when i is out of range).  Context 0 owns every output of dsx_group_survey_host. */
+dsx_ctx* dsx_group_ctx(dsx_group* g, int i);
+/* How dsx_group_survey_host deals the frames: device r extracts frames [first[r], first[r+1]) (first: n_devices + 1
+ * entries).  image_counts (n_devices entries) NULL = as equal as possible, the first n_images % n_devices devices one
+ * frame more.  DSX_ERR_INVALID when an entry is negative or the entries do not sum to n_images.  Host only. */
+int dsx_group_blocks(int n_images, int n_devices, const int32_t* image_counts, int32_t* first);
+/* dsx_survey_host on the group's devices.  Every argument means what it means for dsx_survey_host, and every output lands on
+ * devices[0] in exactly the bytes and order dsx_survey_host on one GPU produces: feats (from dsx_features_alloc on
+ * dsx_group_ctx(g, 0), room for n_images), corr_count, corr_offset, rows6 (device pointers on devices[0]), bbox_out (host).
+ * image_counts: see dsx_group_blocks.  Inside: every device extracts its block of frames (dsx_survey_host without pairs),
+ * the feature blocks are exchanged with cudaMemcpyPeerAsync, device r matches the r-th contiguous block of the pair list
+ * (dsx_match_pairs_peer) and rank 0 collects the rows in pair order (dsx_peer_collect).
+ * k_total non-NULL: the call synchronises, stores the row total and reports DSX_ERR_CAPACITY (or a peer error).  k_total
+ * NULL: the call returns once everything is enqueued; the outputs are ordered on context 0's stream (a blocking stream, so
+ * work on the legacy default stream of devices[0] follows it), the whole cap_rows rows of rows6 are written (the total is
+ * known on the device only: corr_offset[n_pairs]), and dsx_check_error on the group's contexts reports an overflow.
+ * Calls may follow each other without synchronisation; the group keeps the peer protocol's ordering itself.  The peer
+ * blocks are rebuilt when a call brings more pairs or another cap_rows than the previous one. */
+int dsx_group_survey_host(dsx_group* g, const uint8_t* images, const uint8_t* masks, int n_images, int rows, int cols,
+                          size_t step, size_t img_stride, const double* pose6, const double* g_range, int n_range,
+                          const int32_t* img_id, const int32_t* pairs, int n_pairs, const int32_t* image_counts,
+                          dsx_features_dev* feats, int32_t* corr_count, int32_t* corr_offset, double* rows6,
+                          int64_t cap_rows, int64_t* k_total, double* bbox_out);
+
+/* ------------------------------------------------------------------------------------------------
  * The reference's on-disk formats (SURVEY.md section 8f rank 4; host code, no device work), so that test_demo's inputs
  * load without OpenCV / Boost.  Util::LoadInputData, src/util/util.cpp:85-210.
  * ---------------------------------------------------------------------------------------------- */
