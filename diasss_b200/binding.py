@@ -52,9 +52,9 @@ EXPORTS = [
     "dsx_features_free", "dsx_detect_feature_batch_dev", "dsx_detect_feature_batch", "dsx_geo_model_build", "dsx_geo_model_build_batch", "dsx_georef_batch_dev",
     "dsx_match_pairs_dev", "dsx_survey", "dsx_frame_prepare_batch_dev", "dsx_compute_intersection", "dsx_build_pair_list", "dsx_check_error", "dsx_launch_count", "dsx_timing_enable", "dsx_timing_read", "dsx_stage_name", "dsx_popc_peak",
     "dsx_peer_create", "dsx_peer_connect", "dsx_peer_connect_local", "dsx_match_pairs_peer", "dsx_peer_collect", "dsx_peer_destroy",
-    "dsx_group_create", "dsx_group_destroy", "dsx_group_ctx", "dsx_group_blocks", "dsx_group_survey_host",
+    "dsx_group_create", "dsx_group_destroy", "dsx_group_ctx", "dsx_group_blocks", "dsx_group_survey_host", "dsx_group_survey_raw_host",
     "dsx_io_read_matrix", "dsx_io_write_matrix", "dsx_io_read_column",
-    "dsx_debug_level_image", "dsx_debug_candidates", "dsx_debug_level_keys", "dsx_debug_match", "dsx_debug_sincosf", "dsx_debug_fast_profile", "dsx_survey_host", "dsx_get_kps_pairs_dev",
+    "dsx_debug_level_image", "dsx_debug_candidates", "dsx_debug_level_keys", "dsx_debug_match", "dsx_debug_sincosf", "dsx_debug_fast_profile", "dsx_survey_host", "dsx_survey_raw_host", "dsx_get_kps_pairs_dev",
 ]
 
 _lib = None
@@ -311,6 +311,22 @@ class Context:
                                    _p(bbox_out) if bbox_out is not None else C.c_void_p(0)))
         return kt.value if sync else None
 
+    def survey_raw_host(self, raw_ptr, n_images, rows, cols, raw_pitch, raw_stride, poses, g_ranges, img_id, pairs, feats,
+                        corr_count_ptr, corr_offset_ptr, rows6_ptr, cap_rows, sync=True, bbox_out=None, norm_out=None, mask_out=None,
+                        stats_out=None):
+        """dsx_survey_raw_host: survey_host() from raw float64 frames (host or device; pitch and stride in doubles), each
+        frame normalised and masked inside the pipeline.  norm_out / mask_out ([n, rows, cols] u8) and stats_out ([n, 3]
+        f64) are optional host outputs (numpy arrays or raw addresses; page-locked memory keeps their copies asynchronous)."""
+        img_id = np.ascontiguousarray(img_id, np.int32)
+        pairs = np.ascontiguousarray(pairs, np.int32).reshape(-1, 2)
+        assert poses.dtype == np.float64 and poses.flags.c_contiguous and g_ranges.dtype == np.float64 and g_ranges.flags.c_contiguous
+        kt = C.c_int64()
+        _chk(lib().dsx_survey_raw_host(self._h, _p(raw_ptr), n_images, rows, cols, C.c_size_t(raw_pitch), C.c_size_t(raw_stride), _p(poses),
+                                       _p(g_ranges), g_ranges.shape[1], _p(img_id), _p(pairs), len(pairs), C.byref(feats), _p(corr_count_ptr),
+                                       _p(corr_offset_ptr), _p(rows6_ptr), C.c_int64(cap_rows), C.byref(kt) if sync else C.c_void_p(0),
+                                       _p(bbox_out), _p(norm_out), _p(mask_out), _p(stats_out)))
+        return kt.value if sync else None
+
     def survey(self, images_ptr, masks_ptr, n_images, rows, cols, step, img_stride, rowtab_ptr, g_range_ptr, n_range, img_id, bbox,
                pairs, feats, corr_count_ptr, corr_offset_ptr, rows6_ptr, cap_rows, sync=True):
         """dsx_survey: extraction (host or device images), geo look-ups and matching of every listed pair, pipelined."""
@@ -433,6 +449,25 @@ class Group:
                                          _p(pairs), len(pairs), _p(counts), C.byref(feats), _p(corr_count_ptr), _p(corr_offset_ptr),
                                          _p(rows6_ptr), C.c_int64(cap_rows), C.byref(kt) if sync else C.c_void_p(0),
                                          _p(bbox_out) if bbox_out is not None else C.c_void_p(0)))
+        return kt.value if sync else None
+
+    def survey_raw_host(self, raw_ptr, n_images, rows, cols, raw_pitch, raw_stride, poses, g_ranges, img_id, pairs, feats,
+                        corr_count_ptr, corr_offset_ptr, rows6_ptr, cap_rows, image_counts=None, sync=True, bbox_out=None, norm_out=None,
+                        mask_out=None, stats_out=None):
+        """dsx_group_survey_raw_host: Context.survey_raw_host on every device of the group, outputs on devices[0] and in
+        the host blocks."""
+        img_id = np.ascontiguousarray(img_id, np.int32)
+        pairs = np.ascontiguousarray(pairs, np.int32).reshape(-1, 2)
+        counts = None if image_counts is None else np.ascontiguousarray(image_counts, np.int32)
+        if counts is not None and len(counts) != len(self.devices):
+            raise DsxError(ERR_INVALID, "image_counts needs one entry per device")
+        assert poses.dtype == np.float64 and poses.flags.c_contiguous and g_ranges.dtype == np.float64 and g_ranges.flags.c_contiguous
+        kt = C.c_int64()
+        _chk(lib().dsx_group_survey_raw_host(self._h, _p(raw_ptr), n_images, rows, cols, C.c_size_t(raw_pitch), C.c_size_t(raw_stride),
+                                             _p(poses), _p(g_ranges), g_ranges.shape[1], _p(img_id), _p(pairs), len(pairs), _p(counts),
+                                             C.byref(feats), _p(corr_count_ptr), _p(corr_offset_ptr), _p(rows6_ptr), C.c_int64(cap_rows),
+                                             C.byref(kt) if sync else C.c_void_p(0), _p(bbox_out), _p(norm_out), _p(mask_out),
+                                             _p(stats_out)))
         return kt.value if sync else None
 
     def check_error(self):

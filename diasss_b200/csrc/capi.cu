@@ -107,12 +107,23 @@ static PtrInfo classify_ptr(const void* p) {
     return {0, nullptr};
 }
 
+// Raw CV_64F frames that the pipeline prepares itself (dsx_survey_raw_host): Frame::GetNormalizeSSS and GetFilteredMask
+// run on every chunk right behind its copy, into u8 planes staged with the chunk.  pitch / stride in doubles.  The host
+// outputs are optional: norm / mask planes (n x rows x cols u8, contiguous) and {mean, min, max} per frame.
+struct RawFrames {
+    const double* raw; size_t pitch, stride;
+    uint8_t* norm_out; uint8_t* mask_out; double* stats_out;
+};
+
 // Host images -> device feature block, transfer overlapped with extraction (see dsx_detect_feature_batch in the header).
 // `after_chunk(first image, images)` (optional) is called on the host right after a chunk's extraction has been enqueued.
+// With `raw`, the input is raw frames instead of `images` / `masks` (both null): each chunk is copied as doubles (or read
+// in place when device-resident) and prepared into the staging buffer's u8 planes on its extraction lane.
 static int extract_host_pipelined(dsx_ctx* ctx, const uint8_t* images, const uint8_t* masks, int n_images, int rows, int cols,
                                   size_t step, size_t img_stride, dsx_features_dev* out,
-                                  const std::function<int(int, int, cudaEvent_t, cudaStream_t)>& after_chunk = nullptr) {
-    const PtrInfo pi = classify_ptr(images);
+                                  const std::function<int(int, int, cudaEvent_t, cudaStream_t)>& after_chunk = nullptr,
+                                  const RawFrames* raw = nullptr) {
+    const PtrInfo pi = classify_ptr(raw ? (const void*)raw->raw : (const void*)images);
     const PtrInfo pm = masks ? classify_ptr(masks) : PtrInfo{2, nullptr};
     constexpr int NB = dsx_ctx::kPipeBufs;
     if (!ctx->copy_stream) {
@@ -124,7 +135,7 @@ static int extract_host_pipelined(dsx_ctx* ctx, const uint8_t* images, const uin
         if (!ctx->pipe_start) DSX_CUDA(cudaEventCreateWithFlags(&ctx->pipe_start, cudaEventDisableTiming));
         if (!ctx->pipe_join) DSX_CUDA(cudaEventCreateWithFlags(&ctx->pipe_join, cudaEventDisableTiming));
     }
-    if (pi.kind == 2 && pm.kind != 0) {   // nothing to copy
+    if (!raw && pi.kind == 2 && pm.kind != 0) {   // nothing to copy
         if (!after_chunk)
             return extract_chunked(ctx, pi.dev, masks ? pm.dev : nullptr, n_images, rows, cols, step, img_stride, step, img_stride,
                                    out->kps, out->desc, out->count, out->cap);
@@ -143,10 +154,16 @@ static int extract_host_pipelined(dsx_ctx* ctx, const uint8_t* images, const uin
         }
         return DSX_OK;
     }
+    // copy_img: the input planes (u8 images, or raw doubles) cross PCIe; stage_img / stage_mask: the u8 planes extraction
+    // reads sit in the staging buffer (copied there, or prepared there from raw frames)
     const bool copy_img = pi.kind != 2, copy_mask = masks && pm.kind == 0;
+    const bool stage_img = copy_img || raw, stage_mask = copy_mask || raw;
     const size_t pitch = ((size_t)cols + 15) & ~(size_t)15, plane = pitch * rows;
     const int chunk = std::max(1, std::min(ctx->p.h2d_chunk > 0 ? ctx->p.h2d_chunk : 4, n_images));
-    const size_t per_buf = plane * chunk * ((copy_img ? 1 : 0) + (copy_mask ? 1 : 0));
+    // raw input: a buffer holds the chunk's f64 planes (tightly packed; none when they are device-resident), then its
+    // norm and mask planes
+    const size_t raw_plane = (size_t)rows * cols, raw_bytes = raw && copy_img ? (sizeof(double) * raw_plane * chunk + 255) & ~(size_t)255 : 0;
+    const size_t per_buf = raw_bytes + plane * chunk * ((stage_img ? 1 : 0) + (stage_mask ? 1 : 0));
     if (ctx->pipe_bytes < per_buf) {
         DSX_CUDA(cudaDeviceSynchronize());
         for (int b = 0; b < NB; b++) {
@@ -168,6 +185,8 @@ static int extract_host_pipelined(dsx_ctx* ctx, const uint8_t* images, const uin
             if (!lanes[k]->pipe_join) DSX_CUDA(cudaEventCreateWithFlags(&lanes[k]->pipe_join, cudaEventDisableTiming));
         }
     }
+    // frame preparation's statistics scratch is grown here, not inside the loop (growing it synchronises the lane's stream)
+    for (int k = 0; k < n_lanes && raw; k++) DSX_TRY(ensure_prep_scratch(lanes[k], chunk, rows));
     // The OUTPUTS may still be in use by earlier work on the context's stream: the extraction lanes wait for it (lane 0
     // is that stream).  The COPIES do not: a staging buffer is free as soon as the chunk that last used it has been
     // extracted (pipe_free, also across calls), so the next survey's images start crossing PCIe while the previous
@@ -189,11 +208,20 @@ static int extract_host_pipelined(dsx_ctx* ctx, const uint8_t* images, const uin
         nb = sizes[c];
         const int b = c % NB;
         dsx_ctx* L = lanes[c % n_lanes];
-        uint8_t* d_img = ctx->pipe_buf[b];
-        uint8_t* d_mask = d_img + (copy_img ? plane * chunk : 0);
+        double* d_raw = (double*)ctx->pipe_buf[b];
+        uint8_t* d_img = ctx->pipe_buf[b] + raw_bytes;
+        uint8_t* d_mask = d_img + (stage_img ? plane * chunk : 0);
         if (ctx->pipe_free_recorded[b]) DSX_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->pipe_free[b], 0));
         const cudaMemcpyKind kind = cudaMemcpyHostToDevice;
-        if (copy_img) {
+        if (raw && copy_img) {
+            const double* src = raw->raw + (size_t)i0 * raw->stride;
+            if (raw->pitch == (size_t)cols && raw->stride == raw_plane)
+                DSX_CUDA(cudaMemcpyAsync(d_raw, src, sizeof(double) * raw_plane * nb, kind, ctx->copy_stream));
+            else
+                for (int i = 0; i < nb; i++)
+                    DSX_CUDA(cudaMemcpy2DAsync(d_raw + raw_plane * i, sizeof(double) * cols, src + (size_t)i * raw->stride,
+                                               sizeof(double) * raw->pitch, sizeof(double) * cols, rows, kind, ctx->copy_stream));
+        } else if (copy_img) {
             if (step == pitch && img_stride == plane)
                 DSX_CUDA(cudaMemcpyAsync(d_img, images + (size_t)i0 * img_stride, plane * nb, kind, ctx->copy_stream));
             else
@@ -207,10 +235,20 @@ static int extract_host_pipelined(dsx_ctx* ctx, const uint8_t* images, const uin
                                            ctx->copy_stream));
         DSX_CUDA(cudaEventRecord(ctx->pipe_copied[b], ctx->copy_stream));
         DSX_CUDA(cudaStreamWaitEvent(L->stream, ctx->pipe_copied[b], 0));
-        const uint8_t* x_img = copy_img ? d_img : pi.dev + (size_t)i0 * img_stride;
-        const size_t x_step = copy_img ? pitch : step, x_stride = copy_img ? plane : img_stride;
-        const uint8_t* x_mask = !masks ? nullptr : copy_mask ? d_mask : pm.dev + (size_t)i0 * img_stride;
-        const size_t m_step = copy_mask ? pitch : step, m_stride = copy_mask ? plane : img_stride;
+        if (raw) {
+            const double* x_raw = copy_img ? d_raw : (const double*)pi.dev + (size_t)i0 * raw->stride;
+            DSX_TRY(launch_frame_prepare(L, x_raw, nb, rows, cols, copy_img ? (size_t)cols : raw->pitch, copy_img ? raw_plane : raw->stride,
+                                         d_img, d_mask, pitch, plane, raw->stats_out ? raw->stats_out + 3 * (size_t)i0 : nullptr));
+            // the prepared planes leave before pipe_free is recorded below: the buffer is not refilled under the copy
+            // (the planes of consecutive frames are rows at one pitch, so a chunk is one 2-D copy)
+            const size_t o = (size_t)i0 * raw_plane;
+            if (raw->norm_out) DSX_CUDA(cudaMemcpy2DAsync(raw->norm_out + o, cols, d_img, pitch, cols, (size_t)nb * rows, cudaMemcpyDefault, L->stream));
+            if (raw->mask_out) DSX_CUDA(cudaMemcpy2DAsync(raw->mask_out + o, cols, d_mask, pitch, cols, (size_t)nb * rows, cudaMemcpyDefault, L->stream));
+        }
+        const uint8_t* x_img = stage_img ? d_img : pi.dev + (size_t)i0 * img_stride;
+        const size_t x_step = stage_img ? pitch : step, x_stride = stage_img ? plane : img_stride;
+        const uint8_t* x_mask = stage_mask ? d_mask : !masks ? nullptr : pm.dev + (size_t)i0 * img_stride;
+        const size_t m_step = stage_mask ? pitch : step, m_stride = stage_mask ? plane : img_stride;
         DSX_TRY(extract_chunked(L, x_img, x_mask, nb, rows, cols, x_step, x_stride, m_step, m_stride,
                                 out->kps + (size_t)i0 * out->cap, out->desc + (size_t)i0 * out->cap * 32, out->count + i0, out->cap));
         DSX_CUDA(cudaEventRecord(ctx->pipe_free[b], L->stream));      // = "this chunk's features are complete"
@@ -574,7 +612,8 @@ struct GeoHostJob {
 static int survey_impl(dsx_ctx* ctx, const uint8_t* images, const uint8_t* masks, int n_images, int rows, int cols, size_t step,
                        size_t img_stride, const double* d_rowtab6, const double* d_g_range, int n_range, const int32_t* img_id,
                        const double* bbox, GeoHostJob* job, const int32_t* pairs, int n_pairs, dsx_features_dev* feats,
-                       int32_t* corr_count, int32_t* corr_offset, double* rows6, int64_t cap_rows, int64_t* k_total) {
+                       int32_t* corr_count, int32_t* corr_offset, double* rows6, int64_t cap_rows, int64_t* k_total,
+                       const RawFrames* raw = nullptr) {
     // Pairs are matched as soon as both images are extracted: slots = the pair list stably sorted by the later image.
     std::vector<int32_t> order(n_pairs), slot_of(n_pairs), spairs(2 * (size_t)n_pairs), img_rows(n_images, rows);
     for (int p = 0; p < n_pairs; p++) order[p] = p;
@@ -658,7 +697,7 @@ static int survey_impl(dsx_ctx* ctx, const uint8_t* images, const uint8_t* masks
         queued.push_back(Chunk{i0, nb, ev});
         return DSX_OK;
     };
-    int st = extract_host_pipelined(ctx, images, masks, n_images, rows, cols, step, img_stride, &F, after_chunk);
+    int st = extract_host_pipelined(ctx, images, masks, n_images, rows, cols, step, img_stride, &F, after_chunk, raw);
     if (job) {
         for (auto& t : job->pool) t.join();
         job->pool.clear();
@@ -704,12 +743,11 @@ int dsx_survey(dsx_ctx* ctx, const uint8_t* images, const uint8_t* masks, int n_
                        pairs, n_pairs, feats, corr_count, corr_offset, rows6, cap_rows, k_total);
 }
 
-int dsx_survey_host(dsx_ctx* ctx, const uint8_t* images, const uint8_t* masks, int n_images, int rows, int cols, size_t step,
-                    size_t img_stride, const double* pose6, const double* g_range, int n_range, const int32_t* img_id,
-                    const int32_t* pairs, int n_pairs, dsx_features_dev* feats, int32_t* corr_count, int32_t* corr_offset,
-                    double* rows6, int64_t cap_rows, int64_t* k_total, double* bbox_out) {
-    if (!pose6 || !g_range) { set_error("null argument"); return DSX_ERR_INVALID; }
-    DSX_TRY(survey_check(ctx, images, n_images, rows, cols, step, img_stride, img_id, pairs, n_pairs, feats, corr_count, corr_offset, rows6));
+// dsx_survey_host and dsx_survey_raw_host once their arguments are checked: u8 images / masks, or raw frames (`raw`)
+static int survey_host_impl(dsx_ctx* ctx, const uint8_t* images, const uint8_t* masks, const RawFrames* raw, int n_images, int rows,
+                            int cols, size_t step, size_t img_stride, const double* pose6, const double* g_range, int n_range,
+                            const int32_t* img_id, const int32_t* pairs, int n_pairs, dsx_features_dev* feats, int32_t* corr_count,
+                            int32_t* corr_offset, double* rows6, int64_t cap_rows, int64_t* k_total, double* bbox_out) {
     if (cols <= 1 || n_range < cols - cols / 2 + 1) { set_error("geo model: need cols/2+1 ground ranges (SURVEY.md B4)"); return DSX_ERR_INVALID; }
     // staging for the model: pinned host rows (written by the workers) and their device copy, kept with the context
     const size_t need = sizeof(double) * ((size_t)6 * rows + n_range) * n_images;
@@ -748,10 +786,34 @@ int dsx_survey_host(dsx_ctx* ctx, const uint8_t* images, const uint8_t* masks, i
             }
         });
     const int st = survey_impl(ctx, images, masks, n_images, rows, cols, step, img_stride, nullptr, nullptr, n_range, img_id, nullptr, &job,
-                               pairs, n_pairs, feats, corr_count, corr_offset, rows6, cap_rows, k_total);
+                               pairs, n_pairs, feats, corr_count, corr_offset, rows6, cap_rows, k_total, raw);
     for (auto& t : job.pool)          // (an early error return inside leaves the workers running: they reference `job`)
         if (t.joinable()) t.join();
     return st;
+}
+
+int dsx_survey_host(dsx_ctx* ctx, const uint8_t* images, const uint8_t* masks, int n_images, int rows, int cols, size_t step,
+                    size_t img_stride, const double* pose6, const double* g_range, int n_range, const int32_t* img_id,
+                    const int32_t* pairs, int n_pairs, dsx_features_dev* feats, int32_t* corr_count, int32_t* corr_offset,
+                    double* rows6, int64_t cap_rows, int64_t* k_total, double* bbox_out) {
+    if (!pose6 || !g_range) { set_error("null argument"); return DSX_ERR_INVALID; }
+    DSX_TRY(survey_check(ctx, images, n_images, rows, cols, step, img_stride, img_id, pairs, n_pairs, feats, corr_count, corr_offset, rows6));
+    return survey_host_impl(ctx, images, masks, nullptr, n_images, rows, cols, step, img_stride, pose6, g_range, n_range, img_id, pairs,
+                            n_pairs, feats, corr_count, corr_offset, rows6, cap_rows, k_total, bbox_out);
+}
+
+int dsx_survey_raw_host(dsx_ctx* ctx, const double* raw, int n_images, int rows, int cols, size_t raw_pitch, size_t raw_stride,
+                        const double* pose6, const double* g_range, int n_range, const int32_t* img_id, const int32_t* pairs, int n_pairs,
+                        dsx_features_dev* feats, int32_t* corr_count, int32_t* corr_offset, double* rows6, int64_t cap_rows,
+                        int64_t* k_total, double* bbox_out, uint8_t* norm_out, uint8_t* mask_out, double* stats_out) {
+    if (!pose6 || !g_range) { set_error("null argument"); return DSX_ERR_INVALID; }
+    // the raw geometry is checked as the u8 one is, with pitch and stride counted in doubles
+    DSX_TRY(survey_check(ctx, (const uint8_t*)raw, n_images, rows, cols, raw_pitch, raw_stride, img_id, pairs, n_pairs, feats, corr_count,
+                         corr_offset, rows6));
+    if (((uintptr_t)raw & 7) != 0) { set_error("raw must be 8-byte aligned (an array of doubles)"); return DSX_ERR_INVALID; }
+    const RawFrames rf{raw, raw_pitch, raw_stride, norm_out, mask_out, stats_out};
+    return survey_host_impl(ctx, nullptr, nullptr, &rf, n_images, rows, cols, 0, 0, pose6, g_range, n_range, img_id, pairs, n_pairs, feats,
+                            corr_count, corr_offset, rows6, cap_rows, k_total, bbox_out);
 }
 
 int dsx_geo_model_build(const double* pose6, int rows, int cols, const double* g_range, int n_range, double* rowtab6,

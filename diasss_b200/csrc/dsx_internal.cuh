@@ -268,7 +268,9 @@ int launch_finalize(dsx_ctx* ctx, const uint8_t* masks, size_t mstep, size_t mas
                     dsx_keypoint* out_kps, uint8_t* out_desc, int32_t* out_count, int out_cap);
 int launch_georef(dsx_ctx* ctx, const dsx_features_dev* f, const double* rowtab6, const double* g_range, int rows,
                   int cols, int n_range);
-// frameprep.cu : Frame::GetNormalizeSSS + GetFilteredMask
+// frameprep.cu : Frame::GetNormalizeSSS + GetFilteredMask (stats_out: device or host; the scratch for n images can be
+// sized ahead with ensure_prep_scratch, whose growth synchronises the context's stream)
+int ensure_prep_scratch(dsx_ctx* ctx, int n, int rows);
 int launch_frame_prepare(dsx_ctx* ctx, const double* raw, int n, int rows, int cols, size_t raw_pitch, size_t raw_stride,
                          uint8_t* norm, uint8_t* mask, size_t step, size_t img_stride, double* stats_out);
 // match.cu : K7 + K8 + K9

@@ -125,8 +125,7 @@ __global__ void __launch_bounds__(256) prep_map_kernel(const double* __restrict_
 
 }  // namespace
 
-int launch_frame_prepare(dsx_ctx* ctx, const double* raw, int n, int rows, int cols, size_t raw_pitch, size_t raw_stride,
-                         uint8_t* norm, uint8_t* mask, size_t step, size_t img_stride, double* stats_out) {
+int ensure_prep_scratch(dsx_ctx* ctx, int n, int rows) {
     // scratch: [n][rows][3] row statistics + [n][3] image statistics
     const size_t need = sizeof(double) * 3 * ((size_t)n * rows + n);
     if (ctx->prep_scratch_bytes < need) {
@@ -136,6 +135,12 @@ int launch_frame_prepare(dsx_ctx* ctx, const double* raw, int n, int rows, int c
         DSX_CUDA(cudaMalloc(&ctx->prep_scratch, need));
         ctx->prep_scratch_bytes = need;
     }
+    return DSX_OK;
+}
+
+int launch_frame_prepare(dsx_ctx* ctx, const double* raw, int n, int rows, int cols, size_t raw_pitch, size_t raw_stride,
+                         uint8_t* norm, uint8_t* mask, size_t step, size_t img_stride, double* stats_out) {
+    DSX_TRY(ensure_prep_scratch(ctx, n, rows));
     double* rowstat = (double*)ctx->prep_scratch;
     double* imgstat = rowstat + 3 * (size_t)n * rows;
     StageTimer _t(ctx, 9);
@@ -146,7 +151,8 @@ int launch_frame_prepare(dsx_ctx* ctx, const double* raw, int n, int rows, int c
     prep_map_kernel<<<dim3((cols + kPW - 1) / kPW, (rows + kPH - 1) / kPH, n), 256, 0, ctx->stream>>>(
         raw, (long long)raw_pitch, (long long)raw_stride, rows, cols, imgstat, norm, mask, (long long)step, (long long)img_stride);
     DSX_LAUNCH_CHECK();
-    if (stats_out) DSX_CUDA(cudaMemcpyAsync(stats_out, imgstat, sizeof(double) * 3 * n, cudaMemcpyDeviceToDevice, ctx->stream));
+    // stats_out: device memory (dsx_frame_prepare_batch_dev) or host memory (dsx_survey_raw_host)
+    if (stats_out) DSX_CUDA(cudaMemcpyAsync(stats_out, imgstat, sizeof(double) * 3 * n, cudaMemcpyDefault, ctx->stream));
     return DSX_OK;
 }
 

@@ -1,4 +1,4 @@
-// One process, several GPUs: dsx_group_survey_host runs dsx_survey_host on n devices and leaves on devices[0] exactly what
+// One process, several GPUs: dsx_group_survey_host runs dsx_survey_host (dsx_group_survey_raw_host: dsx_survey_raw_host) on n devices and leaves on devices[0] exactly what
 // one context produces for the whole survey (SURVEY.md section 5, "single process, 8 devices ... plain cudaMemcpyPeerAsync").
 // No new kernels: every step is an existing entry point, and this file only orders them across devices.
 //
@@ -113,8 +113,9 @@ struct dsx_group {
     int64_t peer_cap = -1;
     int seq = 0;
     int32_t* h_total = nullptr;              // pinned: row total read back by a synchronous call
-    // shape of the previous call (a call of another shape may grow extraction staging: the group drains first)
-    int last_rows = -1, last_cols = -1, last_range = -1, last_masks = -1;
+    // shape of the previous call (a call of another shape may grow extraction staging: the group drains first); input:
+    // 0 images, 1 images and masks, 2 raw frames
+    int last_rows = -1, last_cols = -1, last_range = -1, last_input = -1;
     std::vector<int> last_counts;
     Workers* workers = nullptr;
 };
@@ -152,6 +153,14 @@ int make_peers(dsx_group* g, int n_pairs, int64_t cap_rows) {
     g->peer_pairs = n_pairs; g->peer_cap = cap_rows;
     return DSX_OK;
 }
+
+// What step 1 extracts from: u8 images and masks (dsx_group_survey_host), or raw frames prepared on the way
+// (dsx_group_survey_raw_host, with its optional host outputs).  pitch / stride in bytes for images, in doubles for raw.
+struct Input {
+    const uint8_t* images; const uint8_t* masks;
+    const double* raw; uint8_t* norm_out; uint8_t* mask_out; double* stats_out;
+    size_t pitch, stride;
+};
 
 dsx_features_dev slice(const dsx_features_dev& f, int first, int count) {
     dsx_features_dev s = f;
@@ -262,15 +271,19 @@ void dsx_group_destroy(dsx_group* g) {
 
 dsx_ctx* dsx_group_ctx(dsx_group* g, int i) { return g && i >= 0 && i < g->n ? g->ctx[i] : nullptr; }
 
-int dsx_group_survey_host(dsx_group* g, const uint8_t* images, const uint8_t* masks, int n_images, int rows, int cols,
-                          size_t step, size_t img_stride, const double* pose6, const double* g_range, int n_range,
-                          const int32_t* img_id, const int32_t* pairs, int n_pairs, const int32_t* image_counts,
-                          dsx_features_dev* feats, int32_t* corr_count, int32_t* corr_offset, double* rows6,
-                          int64_t cap_rows, int64_t* k_total, double* bbox_out) {
+}  // extern "C"
+
+namespace {
+
+int group_survey(dsx_group* g, const Input& in, int n_images, int rows, int cols, const double* pose6, const double* g_range,
+                 int n_range, const int32_t* img_id, const int32_t* pairs, int n_pairs, const int32_t* image_counts,
+                 dsx_features_dev* feats, int32_t* corr_count, int32_t* corr_offset, double* rows6, int64_t cap_rows,
+                 int64_t* k_total, double* bbox_out) {
     using namespace dsx;
-    if (!g || !images || !pose6 || !g_range || !img_id || !feats || !corr_count || !corr_offset || !rows6 || (n_pairs > 0 && !pairs) ||
+    const size_t step = in.pitch, img_stride = in.stride;
+    if (!g || !(in.images || in.raw) || !pose6 || !g_range || !img_id || !feats || !corr_count || !corr_offset || !rows6 || (n_pairs > 0 && !pairs) ||
         n_pairs < 0 || cap_rows < 0) {
-        set_error("dsx_group_survey_host: null or negative argument");
+        set_error("group survey: null or negative argument");
         return DSX_ERR_INVALID;
     }
     const int W = g->n;
@@ -288,10 +301,10 @@ int dsx_group_survey_host(dsx_group* g, const uint8_t* images, const uint8_t* ma
     for (int r = 0; r < W; r++) counts[r] = first[r + 1] - first[r];
 
     // --- set-up that needs an idle group: a new shape (extraction staging may grow), feature blocks, peer blocks
-    const int has_masks = masks ? 1 : 0;
+    const int input = in.raw ? 2 : in.masks ? 1 : 0;
     const bool grow_blocks = [&]() { for (int r = 1; r < W; r++) if (g->blocks[r].n_images < n_images) return true; return false; }();
     const bool new_peers = g->peers.empty() || n_pairs > g->peer_pairs || cap_rows != g->peer_cap;
-    if (rows != g->last_rows || cols != g->last_cols || n_range != g->last_range || has_masks != g->last_masks || counts != g->last_counts ||
+    if (rows != g->last_rows || cols != g->last_cols || n_range != g->last_range || input != g->last_input || counts != g->last_counts ||
         grow_blocks || new_peers) {
         drain(g);
         for (int r = 1; r < W && grow_blocks; r++) {
@@ -307,7 +320,7 @@ int dsx_group_survey_host(dsx_group* g, const uint8_t* images, const uint8_t* ma
             DSX_CUDA(cudaDeviceSynchronize());
         }
         if (new_peers) DSX_TRY(make_peers(g, n_pairs, cap_rows));
-        g->last_rows = rows; g->last_cols = cols; g->last_range = n_range; g->last_masks = has_masks; g->last_counts = counts;
+        g->last_rows = rows; g->last_cols = cols; g->last_range = n_range; g->last_input = input; g->last_counts = counts;
     }
     std::vector<dsx_features_dev> full(W);
     for (int r = 0; r < W; r++) { full[r] = r == 0 ? *feats : g->blocks[r]; full[r].n_images = n_images; }
@@ -325,9 +338,18 @@ int dsx_group_survey_host(dsx_group* g, const uint8_t* images, const uint8_t* ma
             dsx_features_dev mine = slice(full[r], first[r], counts[r]);
             const size_t b = first[r];
             int32_t* sc = (int32_t*)g->scratch[r];
-            DSX_TRY(dsx_survey_host(g->ctx[r], images + b * img_stride, masks ? masks + b * img_stride : nullptr, counts[r], rows, cols, step,
-                                    img_stride, pose6 + b * rows * 6, g_range + b * n_range, n_range, img_id + b, nullptr, 0, &mine, sc,
-                                    sc + 4, (double*)(g->scratch[r] + 128), 0, nullptr, bbox.data() + 4 * b));
+            double* sc_rows = (double*)(g->scratch[r] + 128);
+            if (in.raw) {
+                const size_t px = b * rows * cols;      // this rank's frames of the host outputs
+                DSX_TRY(dsx_survey_raw_host(g->ctx[r], in.raw + b * img_stride, counts[r], rows, cols, step, img_stride, pose6 + b * rows * 6,
+                                            g_range + b * n_range, n_range, img_id + b, nullptr, 0, &mine, sc, sc + 4, sc_rows, 0, nullptr,
+                                            bbox.data() + 4 * b, in.norm_out ? in.norm_out + px : nullptr,
+                                            in.mask_out ? in.mask_out + px : nullptr, in.stats_out ? in.stats_out + 3 * b : nullptr));
+            } else {
+                DSX_TRY(dsx_survey_host(g->ctx[r], in.images + b * img_stride, in.masks ? in.masks + b * img_stride : nullptr, counts[r], rows,
+                                        cols, step, img_stride, pose6 + b * rows * 6, g_range + b * n_range, n_range, img_id + b, nullptr, 0,
+                                        &mine, sc, sc + 4, sc_rows, 0, nullptr, bbox.data() + 4 * b));
+            }
         }
         DSX_CUDA(cudaEventRecord(g->ready[r], s));
         return DSX_OK;
@@ -400,6 +422,31 @@ int dsx_group_survey_host(dsx_group* g, const uint8_t* images, const uint8_t* ma
     DSX_CUDA(cudaStreamSynchronize(s0));
     *k_total = total;
     return DSX_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int dsx_group_survey_host(dsx_group* g, const uint8_t* images, const uint8_t* masks, int n_images, int rows, int cols,
+                          size_t step, size_t img_stride, const double* pose6, const double* g_range, int n_range,
+                          const int32_t* img_id, const int32_t* pairs, int n_pairs, const int32_t* image_counts,
+                          dsx_features_dev* feats, int32_t* corr_count, int32_t* corr_offset, double* rows6,
+                          int64_t cap_rows, int64_t* k_total, double* bbox_out) {
+    const Input in{images, masks, nullptr, nullptr, nullptr, nullptr, step, img_stride};
+    return group_survey(g, in, n_images, rows, cols, pose6, g_range, n_range, img_id, pairs, n_pairs, image_counts, feats, corr_count,
+                        corr_offset, rows6, cap_rows, k_total, bbox_out);
+}
+
+int dsx_group_survey_raw_host(dsx_group* g, const double* raw, int n_images, int rows, int cols, size_t raw_pitch,
+                              size_t raw_stride, const double* pose6, const double* g_range, int n_range,
+                              const int32_t* img_id, const int32_t* pairs, int n_pairs, const int32_t* image_counts,
+                              dsx_features_dev* feats, int32_t* corr_count, int32_t* corr_offset, double* rows6,
+                              int64_t cap_rows, int64_t* k_total, double* bbox_out, uint8_t* norm_out,
+                              uint8_t* mask_out, double* stats_out) {
+    const Input in{nullptr, nullptr, raw, norm_out, mask_out, stats_out, raw_pitch, raw_stride};
+    return group_survey(g, in, n_images, rows, cols, pose6, g_range, n_range, img_id, pairs, n_pairs, image_counts, feats, corr_count,
+                        corr_offset, rows6, cap_rows, k_total, bbox_out);
 }
 
 }  // extern "C"

@@ -7,18 +7,19 @@ Mirrors src/diasss2.cpp:73-97 up to (and excluding) Optimizer::TrajOptimizationA
         pose-xml FileStorage node `auv_pose` (rows x 6 CV_64F)             dsx_io_read_matrix
         altitude / groundrange text files, one number per line             dsx_io_read_column
         annos-xml FileStorage node `anno_kps` (K x 7 CV_32S, optional here: only the back end reads it)
-  Frame::Frame (src/core/frame.cpp:18-55) per image   -> front_end(): GetNormalizeSSS + GetFilteredMask on the device
-        (dsx_frame_prepare_batch_dev), GetGeoImg as the per-ping geo model (dsx_geo_model_build + dsx_georef_batch_dev),
-        DetectFeature (dsx_detect_feature_batch_dev)
-  the i<j loop with Util::ComputeIntersection > MIN_OVERLAP (diasss2.cpp:88-97)  -> dsx_build_pair_list
-  FEAmatcher::RobustMatching per listed pair          -> dsx_match_pairs_dev; rows appended to Source.corres_kps and,
+  Frame::Frame (src/core/frame.cpp:18-55) per image   -> front_end(): one dsx_survey_raw_host call on the raw frames:
+        GetNormalizeSSS + GetFilteredMask on the device behind each chunk's copy, GetGeoImg as the per-ping geo model
+        (dsx_geo_model_build), DetectFeature
+  the i<j loop with Util::ComputeIntersection > MIN_OVERLAP (diasss2.cpp:88-97)  -> dsx_build_pair_list (on the bboxes of
+        dsx_geo_model_build_batch, before the call)
+  FEAmatcher::RobustMatching per listed pair          -> inside the same call; rows appended to Source.corres_kps and,
         mirrored, to Target.corres_kps (FEAmatcher.cpp:35-45) in loop order
 
 write_survey() stores frames in the same formats (the test-suite's stand-in for the reference's unpublished test_data).
 Host I/O only moves bytes; everything numeric runs in libdiasss_b200.so.
 
 CLI:  python -m diasss_b200.demo --image DIR --pose DIR --altitude DIR --groundrange DIR [--annotation DIR] [--out F.npz]
-          [--gpus N]     (N > 1: extraction and matching on devices 0..N-1 of this process, dsx_group_survey_host; same output)
+          [--gpus N]     (N > 1: the same on devices 0..N-1 of this process, dsx_group_survey_raw_host; same output)
 """
 import argparse
 import os
@@ -66,56 +67,35 @@ def write_survey(root, raws, poses, altitudes, granges, annos=None, first_id=170
 
 def front_end(data, device=0, min_overlap=MIN_OVERLAP, gpus=1, **params):
     """Frames + correspondences of a loaded survey (all images of one shape).  Returns dict(frames=[dict(img_id, kps,
-    desc, norm_img, flt_mask, bbox, corres_kps)], pairs, overlap, count, rows6).  gpus > 1: DetectFeature and the matching
-    run on devices 0..gpus-1 (one dsx_group_survey_host call on the host frames); the frames are prepared on `device`."""
+    desc, norm_img, flt_mask, bbox, corres_kps)], pairs, overlap, count, rows6).  One dsx_survey_raw_host call on `device`
+    takes the raw frames from the host and prepares, extracts and matches them; gpus > 1: one dsx_group_survey_raw_host
+    call on devices 0..gpus-1 instead, each device receiving only its own frames."""
     import torch
-    from .frontend import FrontEnd
+    from .frontend import FrontEnd, SurveyGroup
     raws = data["imgs"]
     n = len(raws)
     rows, cols = raws[0].shape
     if any(r.shape != (rows, cols) for r in raws):
         raise ValueError("front_end() batches frames of one shape")
-    dev = torch.device("cuda", device)
-    fe = FrontEnd(device=device, **params)
+    raw = torch.empty((n, rows, cols), dtype=torch.float64, pin_memory=True).numpy()     # page-locked: asynchronous copies
+    np.stack(raws, out=raw)
+    poses = np.stack(data["poses"])
+    n_range = min(len(g) for g in data["granges"])               # (only the first cols/2 + 1 ground ranges are ever read)
+    gr = np.stack([np.asarray(g[:n_range], np.float64) for g in data["granges"]])
+    _, bboxes = B.geo_model_build_batch(poses, rows, cols, gr)   # host threads, same libm calls as the reference
+    pairs, overlap = B.build_pair_list(bboxes, min_overlap)
+    ids = list(range(n))                                         # Frame(i, ...): img_id = position in the sorted list
+    fe = SurveyGroup(list(range(gpus)), **params) if gpus > 1 else FrontEnd(device=device, **params)
     try:
-        step = (cols + 3) & ~3                                   # device images need a row pitch that is a multiple of 4
-        d_raw = torch.from_numpy(np.stack(raws)).to(dev)
-        norm = torch.zeros(n, rows, step, dtype=torch.uint8, device=dev)
-        mask = torch.zeros_like(norm)
-        fe.ctx.frame_prepare_batch_dev(d_raw.data_ptr(), n, rows, cols, norm.data_ptr(), mask.data_ptr(), step=step)
-        del d_raw
-        n_range = min(len(g) for g in data["granges"])           # (only the first cols/2 + 1 ground ranges are ever read)
-        gr = np.stack([np.asarray(g[:n_range], np.float64) for g in data["granges"]])
-        tabs, bboxes = B.geo_model_build_batch(np.stack(data["poses"]), rows, cols, gr)     # host threads, same libm calls as the reference
-        rowtabs = torch.from_numpy(tabs).to(dev)
-        granges = torch.from_numpy(gr).to(dev)
-        pairs, overlap = B.build_pair_list(bboxes, min_overlap)
-        ids = list(range(n))                                     # Frame(i, ...): img_id = position in the sorted list
-        if gpus > 1:
-            from .frontend import SurveyGroup
-            sg = SurveyGroup(list(range(gpus)), **params)
-            try:
-                h_norm = torch.from_numpy(np.ascontiguousarray(norm.cpu().numpy()[:, :, :cols])).pin_memory()
-                h_mask = torch.from_numpy(np.ascontiguousarray(mask.cpu().numpy()[:, :, :cols])).pin_memory()
-                res = sg.process_survey_host(h_norm, h_mask, np.stack(data["poses"]), gr, ids, pairs)
-                feats = res["feats"]
-                if not len(pairs):
-                    res = None
-            finally:
-                sg.close()
-        else:
-            feats = fe.alloc_features(n)
-            fe.ctx.detect_feature_batch_dev(norm.data_ptr(), mask.data_ptr(), n, rows, cols, step, rows * step, feats["c"])
-            fe.ctx.georef_batch_dev(feats["c"], rowtabs.data_ptr(), granges.data_ptr(), rows, cols, n_range)
-            res = fe.match_pairs(feats, ids, [rows] * n, bboxes, pairs) if len(pairs) else None
-        cnt = res["count"].cpu().numpy()[:len(pairs)] if res else np.zeros(0, np.int32)
-        rows6 = res["rows6"].cpu().numpy() if res else np.zeros((0, 6))
+        res = fe.process_survey_raw_host(raw, poses, gr, ids, pairs, prepared=True)
+        feats = res["feats"]
+        cnt = res["count"].cpu().numpy()[:len(pairs)] if len(pairs) else np.zeros(0, np.int32)
+        rows6 = res["rows6"].cpu().numpy() if len(pairs) else np.zeros((0, 6))
         nk = feats["count"].cpu().numpy()
         kps = feats["kps"].cpu().numpy().view(np.uint8).reshape(n, fe.ctx.cap, 28)
         desc = feats["desc"].cpu().numpy()
-        norm_h, mask_h = norm.cpu().numpy()[:, :, :cols], mask.cpu().numpy()[:, :, :cols]
         frames = [dict(img_id=k, kps=kps[k, :nk[k]].copy().view(B.KP_DTYPE).reshape(-1), desc=desc[k, :nk[k]].copy(),
-                       norm_img=norm_h[k], flt_mask=mask_h[k], bbox=bboxes[k], corres_kps=[]) for k in range(n)]
+                       norm_img=res["norm"][k], flt_mask=res["mask"][k], bbox=bboxes[k], corres_kps=[]) for k in range(n)]
         off = 0
         for p, (i, j) in enumerate(pairs):                       # FEAmatcher.cpp:35-45
             r = rows6[off:off + cnt[p]]
@@ -126,7 +106,10 @@ def front_end(data, device=0, min_overlap=MIN_OVERLAP, gpus=1, **params):
             f["corres_kps"] = np.concatenate(f["corres_kps"]) if f["corres_kps"] else np.zeros((0, 6))
         return dict(frames=frames, pairs=pairs, overlap=overlap, count=cnt, rows6=rows6)
     finally:
-        fe.ctx.close()
+        if gpus > 1:
+            fe.close()
+        else:
+            fe.ctx.close()
 
 
 def main(argv=None):

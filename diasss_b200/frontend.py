@@ -11,6 +11,8 @@ Reference interface                                        ->  here
   test_demo's two loops (diasss2.cpp:82-97)                ->  FrontEnd.process_survey (device-resident, batched)
                                                                FrontEnd.process_survey_host (host images and poses in)
                                                                SurveyGroup.process_survey_host (the same on several GPUs)
+  Frame::Frame + the two loops (diasss2.cpp:73-97)         ->  FrontEnd.process_survey_raw_host (raw ct_img frames in)
+                                                               SurveyGroup.process_survey_raw_host (the same on several GPUs)
 
 The C++ twin of this file is include/diasss_b200/shim.hpp.  Everything numeric happens in libdiasss_b200.so (CUDA);
 this module only moves buffers.  torch is used for device memory and streams in the batched path.
@@ -130,8 +132,21 @@ class FrontEnd:
         Returns dict(feats, count[P], offset[P+1], rows6[K,6], k, bbox[F,4]) -- device tensors on this GPU; K and bbox on the host.
         sync=False: nothing is read back (k is None, rows6 is the whole output buffer).
         """
-        return _survey_host(self, lambda *a, **kw: self.ctx.survey_host(*a, **kw), images, masks, poses, g_ranges, img_ids, pairs,
-                            feats, out, sync)
+        F_, rows, cols = images.shape
+        return _survey_host(self, self.ctx.survey_host, (_host_ptr(images), _host_ptr(masks), F_, rows, cols, cols, rows * cols),
+                            images.shape, poses, g_ranges, img_ids, pairs, feats, out, sync)
+
+    def process_survey_raw_host(self, raws, poses, g_ranges, img_ids, pairs, feats=None, out=None, sync=True, prepared=False):
+        """Frame::Frame (GetNormalizeSSS, GetFilteredMask, GetGeoImg) and test_demo's two hot loops from the raw frames
+        (dsx_survey_raw_host): what process_survey_host returns for the frames' norm_img / flt_mask planes.
+
+        raws     : float64 [F, rows, cols] raw ct_img frames: a numpy array or a torch tensor, on the host (pinned or not)
+                   or on this GPU; rows and frames may be padded (unit stride along a row)
+        prepared : also return norm [F, rows, cols] u8, mask [F, rows, cols] u8 and stats [F, 3] ({mean, min, max} of each
+                   raw frame) as numpy arrays in page-locked memory (complete once the call is, or after a synchronise
+                   when sync=False)
+        Everything else as process_survey_host."""
+        return _survey_raw_host(self, self.ctx.survey_raw_host, raws, poses, g_ranges, img_ids, pairs, feats, out, sync, prepared)
 
     def alloc_features(self, n_images):
         """Feature block as torch tensors (so it can be all-gathered with torch.distributed) + its C descriptor."""
@@ -188,8 +203,37 @@ def _host_ptr(a):
     return a.data_ptr()
 
 
-def _survey_host(fe, call, images, masks, poses, g_ranges, img_ids, pairs, feats, out, sync, **kw):
-    F_, rows, cols = images.shape
+def _raw_view(raws):
+    """(address, row pitch, plane stride) of float64 frames [F, rows, cols], pitch and stride in doubles."""
+    if isinstance(raws, np.ndarray):
+        assert raws.dtype == np.float64
+        ptr, strides = raws.ctypes.data, raws.strides
+    else:
+        import torch
+        assert raws.dtype == torch.float64
+        ptr, strides = raws.data_ptr(), tuple(8 * s for s in raws.stride())
+    assert raws.ndim == 3 and strides[2] == 8 and strides[1] % 8 == 0 and strides[0] % 8 == 0
+    return ptr, strides[1] // 8, strides[0] // 8
+
+
+def _survey_raw_host(fe, call, raws, poses, g_ranges, img_ids, pairs, feats, out, sync, prepared, **kw):
+    F_, rows, cols = raws.shape
+    ptr, pitch, stride = _raw_view(raws)
+    host = {}
+    if prepared:
+        import torch
+        host = dict(norm=torch.empty((F_, rows, cols), dtype=torch.uint8, pin_memory=True).numpy(),
+                    mask=torch.empty((F_, rows, cols), dtype=torch.uint8, pin_memory=True).numpy(),
+                    stats=torch.empty((F_, 3), dtype=torch.float64, pin_memory=True).numpy())
+    res = _survey_host(fe, call, (ptr, F_, rows, cols, pitch, stride), raws.shape, poses, g_ranges, img_ids, pairs, feats, out, sync,
+                       norm_out=host.get("norm"), mask_out=host.get("mask"), stats_out=host.get("stats"), **kw)
+    res.update(host)
+    return res
+
+
+def _survey_host(fe, call, inputs, shape, poses, g_ranges, img_ids, pairs, feats, out, sync, **kw):
+    """`call` (Context / Group .survey_host or .survey_raw_host) with its input arguments `inputs` and the rest shared."""
+    F_, rows, cols = shape
     poses = np.ascontiguousarray(poses, np.float64).reshape(F_, rows, 6)
     g_ranges = np.ascontiguousarray(g_ranges, np.float64).reshape(F_, -1)
     pairs = np.ascontiguousarray(pairs, np.int32).reshape(-1, 2)
@@ -198,7 +242,7 @@ def _survey_host(fe, call, images, masks, poses, g_ranges, img_ids, pairs, feats
     if out is None:
         out = fe.alloc_match_out(len(pairs), feats["count"].device)
     bbox = np.zeros((F_, 4), np.float64)
-    k = call(_host_ptr(images), _host_ptr(masks), F_, rows, cols, cols, rows * cols, poses, g_ranges, img_ids, pairs, feats["c"],
+    k = call(*inputs, poses, g_ranges, img_ids, pairs, feats["c"],
              out["count"].data_ptr(), out["offset"].data_ptr(), out["rows6"].data_ptr(), out["rows6"].shape[0], sync=sync,
              bbox_out=bbox, **kw)
     return dict(feats=feats, count=out["count"], offset=out["offset"], rows6=out["rows6"][:k] if sync else out["rows6"], k=k,
@@ -221,9 +265,18 @@ class SurveyGroup(FrontEnd):
         """FrontEnd.process_survey_host on the group's GPUs.  image_counts: frames per device (contiguous blocks in image
         order; None = as equal as possible)."""
         import torch
+        F_, rows, cols = images.shape
         with torch.cuda.device(self.devices[0]):
-            return _survey_host(self, self.group.survey_host, images, masks, poses, g_ranges, img_ids, pairs, feats, out, sync,
-                                image_counts=image_counts)
+            return _survey_host(self, self.group.survey_host, (_host_ptr(images), _host_ptr(masks), F_, rows, cols, cols, rows * cols),
+                                images.shape, poses, g_ranges, img_ids, pairs, feats, out, sync, image_counts=image_counts)
+
+    def process_survey_raw_host(self, raws, poses, g_ranges, img_ids, pairs, feats=None, out=None, sync=True, prepared=False,
+                                image_counts=None):
+        """FrontEnd.process_survey_raw_host on the group's GPUs: each device receives only the raw frames of its block."""
+        import torch
+        with torch.cuda.device(self.devices[0]):
+            return _survey_raw_host(self, self.group.survey_raw_host, raws, poses, g_ranges, img_ids, pairs, feats, out, sync, prepared,
+                                    image_counts=image_counts)
 
     def alloc_features(self, n_images):
         import torch

@@ -2,11 +2,12 @@
 // against the C ABI only -- no OpenCV, no Boost, no GTSAM.  It takes the reference's own command line
 //     test_demo_frontend --image DIR --pose DIR --altitude DIR --groundrange DIR [--annotation DIR] [--out FILE] [--gpus N]
 // loads the folders the way Util::LoadInputData does (files in name order; FileStorage XML nodes ct_img / auv_pose,
-// one-number-per-line text files), builds the frames on the device (GetNormalizeSSS, GetFilteredMask, geo model,
-// DetectFeature), runs the overlap-gated i<j loop with FEAmatcher::RobustMatching and prints the reference's
-// "OVERLAPPING RATE" lines.  --out writes every matched pair's corres_kps rows [id_s id_t y_s x_s y_t x_t] as text.
-// --gpus N (default 1) extracts and matches on devices 0..N-1 of this process with one dsx_group_survey_host call (host
-// images and poses in); the output is the same.
+// one-number-per-line text files), gates the i<j pairs on the frames' geo bounding boxes and prints the reference's
+// "OVERLAPPING RATE" lines, then hands the raw frames to one dsx_survey_raw_host call, which builds the frames on the
+// device (GetNormalizeSSS, GetFilteredMask, geo model, DetectFeature) and runs FEAmatcher::RobustMatching on every
+// listed pair.  --out writes every matched pair's corres_kps rows [id_s id_t y_s x_s y_t x_t] as text.
+// --gpus N (default 1) runs the same on devices 0..N-1 of this process with one dsx_group_survey_raw_host call; the
+// output is the same.
 //
 // Build (see __graft_entry__.build()):
 //   g++ -std=c++11 -O2 examples/test_demo_frontend.cpp -Iinclude -I/usr/local/cuda/include -Ldiasss_b200 -ldiasss_b200
@@ -89,33 +90,18 @@ int main(int argc, char** argv) {
         CK(dsx_io_read_column(f_gr[k].c_str(), granges[k].data(), n, &n));
         n_range = std::min(n_range, n);
     }
-    // --- construct frames (Frame::Frame, frame.cpp:18-55) on the device
+    // --- construct frames (Frame::Frame, frame.cpp:18-55): here only each frame's geo bounding box, which gates the pairs;
+    // GetNormalizeSSS, GetFilteredMask, the geo look-ups and DetectFeature run inside the survey call on the raw frames
     dsx_ctx* ctx = nullptr;
     CK(dsx_create(nullptr, nullptr, &ctx));                                  // ORBextractor(2000, 1.2, 6, 12, 7), frame.cpp:180
-    const size_t step = ((size_t)cols + 3) & ~(size_t)3;
-    double *d_raw = nullptr, *d_rowtab = nullptr, *d_gr = nullptr;
-    uint8_t *d_norm = nullptr, *d_mask = nullptr;
-    CU(cudaMalloc((void**)&d_raw, plane * 8 * F));
-    CU(cudaMalloc((void**)&d_norm, step * rows * F));
-    CU(cudaMalloc((void**)&d_mask, step * rows * F));
-    CU(cudaMemcpy(d_raw, raw.data(), plane * 8 * F, cudaMemcpyHostToDevice));
-    CK(dsx_frame_prepare_batch_dev(ctx, d_raw, F, rows, cols, cols, plane, d_norm, d_mask, step, step * rows, nullptr));
-    std::vector<double> rowtab((size_t)rows * 6 * F), bbox(4 * (size_t)F), gr_packed((size_t)n_range * F);
+    std::vector<double> rowtab((size_t)rows * 6), bbox(4 * (size_t)F), gr_packed((size_t)n_range * F);
     for (int k = 0; k < F; k++) {
-        CK(dsx_geo_model_build(poses.data() + (size_t)rows * 6 * k, rows, cols, granges[k].data(), (int)granges[k].size(),
-                               rowtab.data() + (size_t)rows * 6 * k, bbox.data() + 4 * k));
+        CK(dsx_geo_model_build(poses.data() + (size_t)rows * 6 * k, rows, cols, granges[k].data(), (int)granges[k].size(), rowtab.data(),
+                               bbox.data() + 4 * k));
         std::copy(granges[k].begin(), granges[k].begin() + n_range, gr_packed.begin() + (size_t)n_range * k);
     }
-    CU(cudaMalloc((void**)&d_rowtab, rowtab.size() * 8));
-    CU(cudaMalloc((void**)&d_gr, gr_packed.size() * 8));
-    CU(cudaMemcpy(d_rowtab, rowtab.data(), rowtab.size() * 8, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(d_gr, gr_packed.data(), gr_packed.size() * 8, cudaMemcpyHostToDevice));
     dsx_features_dev feats;
     CK(dsx_features_alloc(ctx, F, &feats));
-    if (gpus == 1) {
-        CK(dsx_detect_feature_batch_dev(ctx, d_norm, d_mask, F, rows, cols, step, step * rows, &feats));
-        CK(dsx_georef_batch_dev(ctx, &feats, d_rowtab, d_gr, rows, cols, n_range));
-    }
     // --- find correspondences between each pair of frames (diasss2.cpp:88-97)
     const int all_pairs = F * (F - 1) / 2;
     std::vector<int32_t> pairs(2 * (size_t)std::max(all_pairs, 1));
@@ -125,7 +111,7 @@ int main(int argc, char** argv) {
     for (int i = 0, q = 0; i < F; i++)
         for (int j = i + 1; j < F; j++, q++)
             printf("The OVERLAPPING RATE Between image %d and %d : %g ...\n", i, j, overlap[q]);
-    std::vector<int32_t> img_id(F), img_rows(F, rows), cnt(std::max(n_pairs, 1)), off(n_pairs + 1, 0);
+    std::vector<int32_t> img_id(F), cnt(std::max(n_pairs, 1)), off(n_pairs + 1, 0);
     for (int k = 0; k < F; k++) img_id[k] = k;                              // Frame(i, ...): img_id = position in the list
     const int64_t cap_rows = (int64_t)std::max(n_pairs, 1) * 2 * dsx_max_keypoints(ctx);
     int32_t *d_cnt = nullptr, *d_off = nullptr;
@@ -135,23 +121,20 @@ int main(int argc, char** argv) {
     CU(cudaMalloc((void**)&d_rows6, sizeof(double) * 6 * cap_rows));
     int64_t k_total = 0;
     dsx_group* group = nullptr;
-    uint8_t *h_norm = nullptr, *h_mask = nullptr;
     if (gpus > 1) {
-        // the same two loops on devices 0..gpus-1: frames in contiguous blocks per device, features exchanged over peer
-        // copies, the pair list cut into blocks, rows collected in pair order on device 0 (where feats and d_rows6 live)
+        // the same on devices 0..gpus-1: each device receives and prepares the raw frames of its contiguous block, features
+        // are exchanged over peer copies, the pair list is cut into blocks, rows are collected in pair order on device 0
+        // (where feats and d_rows6 live)
         std::vector<int> devices(gpus);
         for (int d = 0; d < gpus; d++) devices[d] = d;
         CK(dsx_group_create(nullptr, devices.data(), gpus, &group));
-        CU(cudaMallocHost((void**)&h_norm, step * rows * F));
-        CU(cudaMallocHost((void**)&h_mask, step * rows * F));
-        CU(cudaMemcpy(h_norm, d_norm, step * rows * F, cudaMemcpyDeviceToHost));
-        CU(cudaMemcpy(h_mask, d_mask, step * rows * F, cudaMemcpyDeviceToHost));
-        CK(dsx_group_survey_host(group, h_norm, h_mask, F, rows, cols, step, step * rows, poses.data(), gr_packed.data(), n_range,
-                                 img_id.data(), pairs.data(), n_pairs, nullptr, &feats, d_cnt, d_off, d_rows6, cap_rows, &k_total,
-                                 nullptr));
-    } else if (n_pairs > 0)
-        CK(dsx_match_pairs_dev(ctx, &feats, img_id.data(), img_rows.data(), bbox.data(), pairs.data(), n_pairs, d_cnt, d_off, d_rows6,
-                               cap_rows, &k_total));
+        CK(dsx_group_survey_raw_host(group, raw.data(), F, rows, cols, cols, plane, poses.data(), gr_packed.data(), n_range, img_id.data(),
+                                     pairs.data(), n_pairs, nullptr, &feats, d_cnt, d_off, d_rows6, cap_rows, &k_total, nullptr, nullptr,
+                                     nullptr, nullptr));
+    } else {
+        CK(dsx_survey_raw_host(ctx, raw.data(), F, rows, cols, cols, plane, poses.data(), gr_packed.data(), n_range, img_id.data(),
+                               pairs.data(), n_pairs, &feats, d_cnt, d_off, d_rows6, cap_rows, &k_total, nullptr, nullptr, nullptr, nullptr));
+    }
     std::vector<double> rows6(6 * (size_t)std::max<int64_t>(k_total, 1));
     if (k_total > 0) {
         CU(cudaMemcpy(rows6.data(), d_rows6, sizeof(double) * 6 * k_total, cudaMemcpyDeviceToHost));
@@ -172,8 +155,8 @@ int main(int argc, char** argv) {
         fclose(f);
     }
     dsx_features_free(&feats);
-    cudaFree(d_raw); cudaFree(d_norm); cudaFree(d_mask); cudaFree(d_rowtab); cudaFree(d_gr); cudaFree(d_cnt); cudaFree(d_off); cudaFree(d_rows6);
-    if (group) { dsx_group_destroy(group); cudaFreeHost(h_norm); cudaFreeHost(h_mask); }
+    cudaFree(d_cnt); cudaFree(d_off); cudaFree(d_rows6);
+    if (group) dsx_group_destroy(group);
     dsx_destroy(ctx);
     return 0;
 }

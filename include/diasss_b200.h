@@ -281,6 +281,30 @@ int dsx_survey_host(dsx_ctx* ctx, const uint8_t* images, const uint8_t* masks, i
                     const int32_t* pairs, int n_pairs, dsx_features_dev* feats, int32_t* corr_count, int32_t* corr_offset,
                     double* rows6, int64_t cap_rows, int64_t* k_total, double* bbox_out);
 
+/* dsx_survey_host from the raw images, for a caller that holds what Util::LoadInputData returns: n_images CV_64F ct_img
+ * planes of rows x cols (row pitch raw_pitch, plane stride raw_stride, both in doubles, as for
+ * dsx_frame_prepare_batch_dev).  raw may be pageable host, page-locked host or device memory (device memory is read in
+ * place).  Each frame goes through Frame::Frame's GetNormalizeSSS + GetFilteredMask (the kernels of
+ * dsx_frame_prepare_batch_dev) inside the pipeline: every chunk of raw frames is prepared on the device right behind its
+ * copy and extracted from the prepared planes, so the preparation overlaps the transfer of the next chunks.  The
+ * outputs are byte-identical to dsx_frame_prepare_batch_dev on the same frames followed by dsx_survey_host on the planes
+ * it produced.  Every other argument means what it means for dsx_survey_host.
+ * Optional host outputs (NULL = not produced; asking for them changes no other output):
+ *   norm_out   Frame::norm_img, n_images x rows x cols u8, contiguous
+ *   mask_out   Frame::flt_mask, same layout
+ *   stats_out  {mean, min, max} of each raw frame, n_images x 3 doubles
+ * They are copied out chunk by chunk while the survey runs; in page-locked memory the copies are asynchronous, in
+ * pageable memory each chunk's copy holds the calling thread until it is done.
+ * Synchronisation as dsx_survey_host: k_total given, the call synchronises and every output is complete on return;
+ * k_total NULL, the host outputs are complete once the work the call ordered on the context's stream is complete.
+ * Device staging: 10 bytes per pixel per frame of a chunk (h2d_chunk frames, default 4) for each of the pipeline's
+ * 4 buffers; 2 bytes per pixel when raw is device memory. */
+int dsx_survey_raw_host(dsx_ctx* ctx, const double* raw, int n_images, int rows, int cols, size_t raw_pitch,
+                        size_t raw_stride, const double* pose6, const double* g_range, int n_range,
+                        const int32_t* img_id, const int32_t* pairs, int n_pairs, dsx_features_dev* feats,
+                        int32_t* corr_count, int32_t* corr_offset, double* rows6, int64_t cap_rows, int64_t* k_total,
+                        double* bbox_out, uint8_t* norm_out, uint8_t* mask_out, double* stats_out);
+
 /* ------------------------------------------------------------------------------------------------
  * Multi-GPU collection over peer memory (one process per GPU; SURVEY.md section 8e).  The pair list of the i<j loop
  * (src/diasss2.cpp:88-97) is cut into `world` contiguous blocks; rank r matches block r and writes its rows
@@ -347,6 +371,16 @@ int dsx_group_survey_host(dsx_group* g, const uint8_t* images, const uint8_t* ma
                           const int32_t* img_id, const int32_t* pairs, int n_pairs, const int32_t* image_counts,
                           dsx_features_dev* feats, int32_t* corr_count, int32_t* corr_offset, double* rows6,
                           int64_t cap_rows, int64_t* k_total, double* bbox_out);
+/* dsx_survey_raw_host on the group's devices, as dsx_group_survey_host is dsx_survey_host: device r receives only the
+ * raw bytes of its own frames [first[r], first[r+1]) and prepares them behind the copy.  Every output lands on devices[0],
+ * or in the host blocks, in exactly the bytes of the one-GPU call; device r writes norm_out, mask_out and stats_out of its
+ * own frames.  k_total NULL: the host outputs are complete once context 0's stream has run what the call ordered. */
+int dsx_group_survey_raw_host(dsx_group* g, const double* raw, int n_images, int rows, int cols, size_t raw_pitch,
+                              size_t raw_stride, const double* pose6, const double* g_range, int n_range,
+                              const int32_t* img_id, const int32_t* pairs, int n_pairs, const int32_t* image_counts,
+                              dsx_features_dev* feats, int32_t* corr_count, int32_t* corr_offset, double* rows6,
+                              int64_t cap_rows, int64_t* k_total, double* bbox_out, uint8_t* norm_out,
+                              uint8_t* mask_out, double* stats_out);
 
 /* ------------------------------------------------------------------------------------------------
  * The reference's on-disk formats (SURVEY.md section 8f rank 4; host code, no device work), so that test_demo's inputs
