@@ -53,7 +53,7 @@ EXPORTS = [
     "dsx_match_pairs_dev", "dsx_survey", "dsx_frame_prepare_batch_dev", "dsx_compute_intersection", "dsx_build_pair_list", "dsx_check_error", "dsx_launch_count", "dsx_timing_enable", "dsx_timing_read", "dsx_stage_name", "dsx_popc_peak",
     "dsx_peer_create", "dsx_peer_connect", "dsx_peer_connect_local", "dsx_match_pairs_peer", "dsx_peer_collect", "dsx_peer_destroy",
     "dsx_group_create", "dsx_group_destroy", "dsx_group_ctx", "dsx_group_blocks", "dsx_group_survey_host", "dsx_group_survey_raw_host",
-    "dsx_io_read_matrix", "dsx_io_write_matrix", "dsx_io_read_column",
+    "dsx_io_read_matrix", "dsx_io_write_matrix", "dsx_io_read_column", "dsx_io_read_matrix_batch",
     "dsx_debug_level_image", "dsx_debug_candidates", "dsx_debug_level_keys", "dsx_debug_match", "dsx_debug_sincosf", "dsx_debug_fast_profile", "dsx_survey_host", "dsx_survey_raw_host", "dsx_get_kps_pairs_dev",
 ]
 
@@ -340,6 +340,24 @@ class Context:
                               C.c_int64(cap_rows), C.byref(kt) if sync else C.c_void_p(0)))
         return kt.value if sync else None
 
+    def io_read_matrix_batch(self, paths, node, out):
+        """dsx_io_read_matrix_batch: the CV_64F node `node` of every file into out[k], the decimal text converted on this
+        context's GPU.  out: float64 [F, rows, cols] numpy array or torch tensor, on this GPU or in host memory (pageable or
+        page-locked), rows and planes may be padded.  Every value is bit for bit io_read_matrix's.  Returns how many values
+        were converted on the host."""
+        if isinstance(out, np.ndarray):
+            ptr, strides, dtype_ok = out.ctypes.data, out.strides, out.dtype == np.float64
+        else:
+            import torch
+            ptr, strides, dtype_ok = out.data_ptr(), tuple(8 * s for s in out.stride()), out.dtype == torch.float64
+        if not dtype_ok or out.ndim != 3 or len(paths) != out.shape[0] or strides[2] != 8 or strides[1] % 8 or strides[0] % 8:
+            raise DsxError(ERR_INVALID, "out must be float64 [len(paths), rows, cols] with unit column stride")
+        arr = (C.c_char_p * max(len(paths), 1))(*[os.fsencode(p) for p in paths])
+        hv = C.c_int64()
+        _chk(lib().dsx_io_read_matrix_batch(self._h, arr, len(paths), node.encode(), int(out.shape[1]), int(out.shape[2]), C.c_void_p(ptr),
+                                            C.c_size_t(strides[1] // 8), C.c_size_t(strides[0] // 8), C.byref(hv)))
+        return hv.value
+
     def check_error(self):
         _chk(lib().dsx_check_error(self._h))
 
@@ -489,6 +507,13 @@ class Group:
 
 
 _DT = {"d": np.float64, "f": np.float32, "i": np.int32, "s": np.int16, "w": np.uint16, "u": np.uint8, "c": np.int8}
+
+
+def io_matrix_shape(path, node):
+    """(rows, cols, element type letter) of one opencv-matrix node: dsx_io_read_matrix's size query."""
+    r, c, dt = C.c_int(), C.c_int(), C.c_char()
+    _chk(lib().dsx_io_read_matrix(os.fsencode(path), node.encode(), C.byref(r), C.byref(c), C.byref(dt), C.c_void_p(0), C.c_size_t(0)))
+    return r.value, c.value, dt.value.decode()
 
 
 def io_read_matrix(path, node):

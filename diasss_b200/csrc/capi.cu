@@ -457,6 +457,7 @@ void dsx_destroy(dsx_ctx* ctx) {
     if (ctx->geo_copied) cudaEventDestroy(ctx->geo_copied);
     if (ctx->kp_scratch) cudaFree(ctx->kp_scratch);
     for (cudaEvent_t e : ctx->chunk_events) cudaEventDestroy(e);
+    free_xml_stage(ctx);
     delete ctx;
 }
 

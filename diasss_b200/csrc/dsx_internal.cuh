@@ -8,6 +8,7 @@
 #include <atomic>
 
 #include <string>
+#include <string_view>
 #include <vector>
 
 #include "../../include/diasss_b200.h"
@@ -23,6 +24,7 @@ constexpr int kMaxDim = 32760;    // coordinates are packed in 16 bits
 constexpr unsigned long long kBestOrderMask = 0x00ffffffffffffffull;
 
 void set_error(const std::string& s);
+struct XmlStage;                  // xmlparse.cu: dsx_io_read_matrix_batch's staging, cached in the context
 extern std::atomic<int64_t> g_launches;   // kernels launched (several host threads launch at once)
 
 #define DSX_CUDA(expr)                                                                             \
@@ -219,6 +221,7 @@ struct dsx_ctx {
     cudaEvent_t geo_copied = nullptr; bool geo_copy_pending = false;               // ... and "its copy to the device has run"
     int32_t* kp_scratch = nullptr; size_t kp_scratch_ints = 0;                         // dsx_get_kps_pairs_dev: pair list + image ids
     std::vector<cudaEvent_t> chunk_events;                                          // dsx_survey_host: markers of deferred chunks
+    dsx::XmlStage* xml = nullptr;                                                   // dsx_io_read_matrix_batch: staging slots, text and parse buffers
     static constexpr int kPipeBufs = 4;
     uint8_t* pipe_buf[kPipeBufs] = {nullptr}; size_t pipe_bytes = 0;
     bool pipe_free_recorded[kPipeBufs] = {false};
@@ -290,6 +293,25 @@ int peer_wait_and_scan(dsx_ctx* ctx, const unsigned* done, int world, unsigned s
 int launch_hamming(dsx_ctx* ctx, const uint8_t* a, const uint8_t* b, int n, int32_t* out);
 int launch_consistent_check(dsx_ctx* ctx, const int32_t* c1, const int32_t* c2, int ns, int nt, int inl1, int inl2, double m1, double m2,
                             bool flipped, int rows_s, int rows_t, int32_t* out, int32_t* out_count);
+
+// io.cu : the FileStorage XML format, shared by dsx_io_read_matrix and dsx_io_read_matrix_batch (xmlparse.cu).  The text
+// handed to these must be followed by a NUL byte (strtol / strtod may look one byte past the element they read).
+struct XmlMatrix {
+    int rows = 0, cols = 0;
+    char dt = 0;
+    bool has_data = false;
+    size_t data_b = 0, data_e = 0;   // text of <data> ... </data>
+};
+bool read_file(const char* path, std::string& out);
+// skips ' ' '\n' '\r' '\t', then reads one value (strtod, or OpenCV's .Inf / -.Inf / .Nan); false if none
+bool parse_number(const char*& p, const char* end, double* v);
+// finds the opencv-matrix node `node` and reads rows / cols / dt and the bounds of <data>; error messages name `path`
+// where dsx_io_read_matrix's do
+int xml_find_matrix(std::string_view s, const char* path, const char* node, XmlMatrix* m);
+// the rows*cols values of <data>, converted to the element type, row-major
+int xml_read_values(std::string_view s, const XmlMatrix& m, void* data);
+// xmlparse.cu : releases the staging of dsx_io_read_matrix_batch
+void free_xml_stage(dsx_ctx* ctx);
 
 // RAII stage timer: records an event pair around a kernel group when timing is enabled.
 struct StageTimer {

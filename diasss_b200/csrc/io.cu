@@ -12,23 +12,12 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <string_view>
 #include <vector>
 
 #include "dsx_internal.cuh"
 
 namespace {
-
-bool read_file(const char* path, std::string& out) {
-    FILE* f = fopen(path, "rb");
-    if (!f) return false;
-    fseek(f, 0, SEEK_END);
-    const long n = ftell(f);
-    fseek(f, 0, SEEK_SET);
-    out.resize(n > 0 ? (size_t)n : 0);
-    const size_t got = n > 0 ? fread(&out[0], 1, (size_t)n, f) : 0;
-    fclose(f);
-    return got == out.size();
-}
 
 int elem_size(char dt) {
     switch (dt) {
@@ -41,14 +30,30 @@ int elem_size(char dt) {
 }
 
 // text between <tag> and </tag> inside [b, e); empty range if absent
-bool inner(const std::string& s, size_t b, size_t e, const char* tag, size_t* ib, size_t* ie) {
+bool inner(std::string_view s, size_t b, size_t e, const char* tag, size_t* ib, size_t* ie) {
     const std::string open = std::string("<") + tag + ">", close = std::string("</") + tag + ">";
     const size_t p = s.find(open, b);
-    if (p == std::string::npos || p >= e) return false;
+    if (p == std::string_view::npos || p >= e) return false;
     const size_t q = s.find(close, p);
-    if (q == std::string::npos || q > e) return false;
+    if (q == std::string_view::npos || q > e) return false;
     *ib = p + open.size(); *ie = q;
     return true;
+}
+
+}  // namespace
+
+namespace dsx {
+
+bool read_file(const char* path, std::string& out) {
+    FILE* f = fopen(path, "rb");
+    if (!f) return false;
+    fseek(f, 0, SEEK_END);
+    const long n = ftell(f);
+    fseek(f, 0, SEEK_SET);
+    out.resize(n > 0 ? (size_t)n : 0);
+    const size_t got = n > 0 ? fread(&out[0], 1, (size_t)n, f) : 0;
+    fclose(f);
+    return got == out.size();
 }
 
 // OpenCV writes special values as .Inf / -.Inf / .Nan
@@ -67,48 +72,43 @@ bool parse_number(const char*& p, const char* end, double* v) {
     return true;
 }
 
-}  // namespace
-
-extern "C" {
-
-int dsx_io_read_matrix(const char* path, const char* node, int* rows, int* cols, char* dt, void* data, size_t cap_bytes) {
-    using namespace dsx;
-    if (!path || !node || !rows || !cols || !dt) { set_error("dsx_io_read_matrix: null argument"); return DSX_ERR_INVALID; }
-    std::string s;
-    if (!read_file(path, s)) { set_error(std::string("cannot read ") + path); return DSX_ERR_INVALID; }
+int xml_find_matrix(std::string_view s, const char* path, const char* node, XmlMatrix* m) {
     // the node's element: <node type_id="opencv-matrix"> ... </node>
-    size_t b = std::string::npos;
+    size_t b = std::string_view::npos;
     const std::string t1 = std::string("<") + node + " ", t2 = std::string("<") + node + ">";
-    for (size_t p = 0; (p = s.find(std::string("<") + node, p)) != std::string::npos; p++)
+    for (size_t p = 0; (p = s.find(std::string("<") + node, p)) != std::string_view::npos; p++)
         if (s.compare(p, t1.size(), t1) == 0 || s.compare(p, t2.size(), t2) == 0) { b = p; break; }
-    const size_t e = b == std::string::npos ? b : s.find(std::string("</") + node + ">", b);
-    if (b == std::string::npos || e == std::string::npos) { set_error(std::string("node '") + node + "' not found in " + path); return DSX_ERR_INVALID; }
+    const size_t e = b == std::string_view::npos ? b : s.find(std::string("</") + node + ">", b);
+    if (b == std::string_view::npos || e == std::string_view::npos) { set_error(std::string("node '") + node + "' not found in " + path); return DSX_ERR_INVALID; }
     const size_t head_end = s.find('>', b);
-    if (s.substr(b, head_end - b).find("opencv-matrix") == std::string::npos) { set_error(std::string("node '") + node + "' is not an opencv-matrix"); return DSX_ERR_INVALID; }
+    if (s.substr(b, head_end - b).find("opencv-matrix") == std::string_view::npos) { set_error(std::string("node '") + node + "' is not an opencv-matrix"); return DSX_ERR_INVALID; }
     size_t ib, ie;
     if (!inner(s, b, e, "rows", &ib, &ie)) { set_error("matrix without <rows>"); return DSX_ERR_INVALID; }
-    const long R = strtol(s.c_str() + ib, nullptr, 10);
+    const long R = strtol(s.data() + ib, nullptr, 10);
     if (!inner(s, b, e, "cols", &ib, &ie)) { set_error("matrix without <cols>"); return DSX_ERR_INVALID; }
-    const long C = strtol(s.c_str() + ib, nullptr, 10);
+    const long C = strtol(s.data() + ib, nullptr, 10);
     if (!inner(s, b, e, "dt", &ib, &ie)) { set_error("matrix without <dt>"); return DSX_ERR_INVALID; }
-    std::string d = s.substr(ib, ie - ib);
+    std::string d(s.substr(ib, ie - ib));
     while (!d.empty() && (d.back() == ' ' || d.back() == '\n')) d.pop_back();
     while (!d.empty() && (d[0] == ' ' || d[0] == '\n' || d[0] == '1')) d.erase(0, 1);      // "1d" = one channel
     if (d.size() != 1 || elem_size(d[0]) == 0 || R < 0 || C < 0 || R > 0x7fffffff || C > 0x7fffffff) {
         set_error("unsupported matrix element type '" + d + "' (single-channel d, f, i, s, w, u, c are read)");
         return DSX_ERR_INVALID;
     }
-    *rows = (int)R; *cols = (int)C; *dt = d[0];
-    if (!data) return DSX_OK;                                  // size query
-    const size_t n = (size_t)R * (size_t)C, es = (size_t)elem_size(d[0]);
-    if (cap_bytes < n * es) { set_error("dsx_io_read_matrix: buffer too small"); return DSX_ERR_CAPACITY; }
-    if (!inner(s, b, e, "data", &ib, &ie)) { if (n == 0) return DSX_OK; set_error("matrix without <data>"); return DSX_ERR_INVALID; }
-    const char* p = s.c_str() + ib;
-    const char* end = s.c_str() + ie;
+    m->rows = (int)R; m->cols = (int)C; m->dt = d[0];
+    m->has_data = inner(s, b, e, "data", &m->data_b, &m->data_e);
+    return DSX_OK;
+}
+
+int xml_read_values(std::string_view s, const XmlMatrix& m, void* data) {
+    const size_t n = (size_t)m.rows * (size_t)m.cols;
+    if (!m.has_data) { if (n == 0) return DSX_OK; set_error("matrix without <data>"); return DSX_ERR_INVALID; }
+    const char* p = s.data() + m.data_b;
+    const char* end = s.data() + m.data_e;
     for (size_t k = 0; k < n; k++) {
         double v;
         if (!parse_number(p, end, &v)) { set_error("matrix data ends after " + std::to_string(k) + " of " + std::to_string(n) + " elements"); return DSX_ERR_INVALID; }
-        switch (d[0]) {
+        switch (m.dt) {
             case 'd': ((double*)data)[k] = v; break;
             case 'f': ((float*)data)[k] = (float)v; break;
             case 'i': ((int32_t*)data)[k] = (int32_t)v; break;
@@ -119,6 +119,24 @@ int dsx_io_read_matrix(const char* path, const char* node, int* rows, int* cols,
         }
     }
     return DSX_OK;
+}
+
+}  // namespace dsx
+
+extern "C" {
+
+int dsx_io_read_matrix(const char* path, const char* node, int* rows, int* cols, char* dt, void* data, size_t cap_bytes) {
+    using namespace dsx;
+    if (!path || !node || !rows || !cols || !dt) { set_error("dsx_io_read_matrix: null argument"); return DSX_ERR_INVALID; }
+    std::string s;
+    if (!read_file(path, s)) { set_error(std::string("cannot read ") + path); return DSX_ERR_INVALID; }
+    XmlMatrix m;
+    DSX_TRY(xml_find_matrix(s, path, node, &m));
+    *rows = m.rows; *cols = m.cols; *dt = m.dt;
+    if (!data) return DSX_OK;                                  // size query
+    const size_t n = (size_t)m.rows * (size_t)m.cols, es = (size_t)elem_size(m.dt);
+    if (cap_bytes < n * es) { set_error("dsx_io_read_matrix: buffer too small"); return DSX_ERR_CAPACITY; }
+    return xml_read_values(s, m, data);
 }
 
 int dsx_io_write_matrix(const char* path, const char* node, int rows, int cols, char dt, const void* data) {

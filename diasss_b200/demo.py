@@ -3,8 +3,9 @@
 Mirrors src/diasss2.cpp:73-97 up to (and excluding) Optimizer::TrajOptimizationAll:
 
   Util::LoadInputData (src/util/util.cpp:44-210)      -> load_input_data(): files of every folder in name order;
-        img-xml  FileStorage node `ct_img`   (CV_64F rows x cols)          dsx_io_read_matrix
-        pose-xml FileStorage node `auv_pose` (rows x 6 CV_64F)             dsx_io_read_matrix
+        img-xml  FileStorage node `ct_img`   (CV_64F rows x cols)          dsx_io_read_matrix, or (parse_device given, as
+        pose-xml FileStorage node `auv_pose` (rows x 6 CV_64F)             main() does) dsx_io_read_matrix_batch: the
+                                                                           decimal text converted on the GPU
         altitude / groundrange text files, one number per line             dsx_io_read_column
         annos-xml FileStorage node `anno_kps` (K x 7 CV_32S, optional here: only the back end reads it)
   Frame::Frame (src/core/frame.cpp:18-55) per image   -> front_end(): one dsx_survey_raw_host call on the raw frames:
@@ -35,10 +36,21 @@ def _sorted_files(folder):
     return [os.path.join(folder, f) for f in sorted(os.listdir(folder)) if os.path.isfile(os.path.join(folder, f))]
 
 
-def load_input_data(image, pose, altitude, groundrange, annotation=None):
-    """Util::LoadInputData: lists of raw images (f64), poses (rows x 6 f64), altitudes, ground ranges, annotations."""
-    data = dict(imgs=[B.io_read_matrix(p, "ct_img") for p in _sorted_files(image)],
-                poses=[B.io_read_matrix(p, "auv_pose") for p in _sorted_files(pose)],
+def load_input_data(image, pose, altitude, groundrange, annotation=None, parse_device=None, frames_on="device"):
+    """Util::LoadInputData: raw images (f64), poses (rows x 6 f64), altitudes, ground ranges, annotations.
+
+    parse_device None (default): every file through dsx_io_read_matrix on the host; imgs and poses are lists of arrays.
+    parse_device = a CUDA ordinal: the ct_img and auv_pose files through dsx_io_read_matrix_batch, their text converted
+    on that GPU (same values, bit for bit).  imgs is then one float64 [F, rows, cols] array: a torch tensor on that GPU
+    (frames_on="device", what dsx_survey_raw_host reads in place) or a page-locked numpy array (frames_on="host", for
+    dsx_group_survey_raw_host); poses are views of one host array [F, rows, 6]."""
+    f_img, f_pose = _sorted_files(image), _sorted_files(pose)
+    if parse_device is None:
+        imgs = [B.io_read_matrix(p, "ct_img") for p in f_img]
+        poses = [B.io_read_matrix(p, "auv_pose") for p in f_pose]
+    else:
+        imgs, poses = _read_batch(f_img, f_pose, parse_device, frames_on)
+    data = dict(imgs=imgs, poses=poses,
                 altitudes=[B.io_read_column(p) for p in _sorted_files(altitude)],
                 granges=[B.io_read_column(p) for p in _sorted_files(groundrange)],
                 annos=[B.io_read_matrix(p, "anno_kps") for p in _sorted_files(annotation)] if annotation else [])
@@ -46,6 +58,31 @@ def load_input_data(image, pose, altitude, groundrange, annotation=None):
     if not (len(data["poses"]) == len(data["altitudes"]) == len(data["granges"]) == n) or (annotation and len(data["annos"]) != n):
         raise ValueError("the input folders hold different numbers of files")
     return data
+
+
+def _read_batch(f_img, f_pose, device, frames_on):
+    import torch
+    if frames_on not in ("device", "host"):
+        raise ValueError("frames_on is 'device' or 'host'")
+    ctx = B.Context(device=device)
+    try:
+        imgs, poses = [], []
+        if f_img:
+            rows, cols, _ = B.io_matrix_shape(f_img[0], "ct_img")
+            shape = (len(f_img), rows, cols)
+            if frames_on == "device":
+                imgs = torch.empty(shape, dtype=torch.float64, device="cuda:%d" % device)
+            else:
+                imgs = torch.empty(shape, dtype=torch.float64, pin_memory=True).numpy()
+            ctx.io_read_matrix_batch(f_img, "ct_img", imgs)
+        if f_pose:
+            rows, cols, _ = B.io_matrix_shape(f_pose[0], "auv_pose")
+            stacked = np.empty((len(f_pose), rows, cols), np.float64)
+            ctx.io_read_matrix_batch(f_pose, "auv_pose", stacked)
+            poses = list(stacked)
+        return imgs, poses
+    finally:
+        ctx.close()
 
 
 def write_survey(root, raws, poses, altitudes, granges, annos=None, first_id=170):
@@ -74,11 +111,15 @@ def front_end(data, device=0, min_overlap=MIN_OVERLAP, gpus=1, **params):
     from .frontend import FrontEnd, SurveyGroup
     raws = data["imgs"]
     n = len(raws)
-    rows, cols = raws[0].shape
-    if any(r.shape != (rows, cols) for r in raws):
-        raise ValueError("front_end() batches frames of one shape")
-    raw = torch.empty((n, rows, cols), dtype=torch.float64, pin_memory=True).numpy()     # page-locked: asynchronous copies
-    np.stack(raws, out=raw)
+    if isinstance(raws, list):
+        rows, cols = raws[0].shape
+        if any(r.shape != (rows, cols) for r in raws):
+            raise ValueError("front_end() batches frames of one shape")
+        raw = torch.empty((n, rows, cols), dtype=torch.float64, pin_memory=True).numpy()     # page-locked: asynchronous copies
+        np.stack(raws, out=raw)
+    else:                                                        # stacked by load_input_data(parse_device=...): used in place
+        raw = raws
+        rows, cols = raw.shape[1:]
     poses = np.stack(data["poses"])
     n_range = min(len(g) for g in data["granges"])               # (only the first cols/2 + 1 ground ranges are ever read)
     gr = np.stack([np.asarray(g[:n_range], np.float64) for g in data["granges"]])
@@ -121,9 +162,10 @@ def main(argv=None):
     ap.add_argument("--device", type=int, default=0)
     ap.add_argument("--gpus", type=int, default=1, help="extract and match on devices 0..N-1 of this process (same output)")
     a = ap.parse_args(argv)
-    data = load_input_data(a.image, a.pose, a.altitude, a.groundrange, a.annotation)
+    data = load_input_data(a.image, a.pose, a.altitude, a.groundrange, a.annotation, parse_device=a.device,
+                           frames_on="device" if a.gpus == 1 else "host")
     for k, im in enumerate(data["imgs"]):
-        print("image size: %d %d" % im.shape)                   # (util.cpp:94)
+        print("image size: %d %d" % tuple(im.shape))            # (util.cpp:94)
     res = front_end(data, device=a.device, gpus=a.gpus)
     q = 0
     n = len(res["frames"])

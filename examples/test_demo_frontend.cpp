@@ -1,11 +1,11 @@
 // test_demo's front end (src/diasss2.cpp:26-97, everything before Optimizer::TrajOptimizationAll) on a B200, written
 // against the C ABI only -- no OpenCV, no Boost, no GTSAM.  It takes the reference's own command line
 //     test_demo_frontend --image DIR --pose DIR --altitude DIR --groundrange DIR [--annotation DIR] [--out FILE] [--gpus N]
-// loads the folders the way Util::LoadInputData does (files in name order; FileStorage XML nodes ct_img / auv_pose,
-// one-number-per-line text files), gates the i<j pairs on the frames' geo bounding boxes and prints the reference's
-// "OVERLAPPING RATE" lines, then hands the raw frames to one dsx_survey_raw_host call, which builds the frames on the
-// device (GetNormalizeSSS, GetFilteredMask, geo model, DetectFeature) and runs FEAmatcher::RobustMatching on every
-// listed pair.  --out writes every matched pair's corres_kps rows [id_s id_t y_s x_s y_t x_t] as text.
+// loads the folders the way Util::LoadInputData does (files in name order; FileStorage XML nodes ct_img / auv_pose, their
+// text converted on the GPU by dsx_io_read_matrix_batch; one-number-per-line text files), gates the i<j pairs on the
+// frames' geo bounding boxes and prints the reference's "OVERLAPPING RATE" lines, then hands the raw frames to one
+// dsx_survey_raw_host call, which builds the frames on the device (GetNormalizeSSS, GetFilteredMask, geo model,
+// DetectFeature) and runs FEAmatcher::RobustMatching on every listed pair.  --out writes every matched pair's corres_kps rows [id_s id_t y_s x_s y_t x_t] as text.
 // --gpus N (default 1) runs the same on devices 0..N-1 of this process with one dsx_group_survey_raw_host call; the
 // output is the same.
 //
@@ -72,18 +72,15 @@ int main(int argc, char** argv) {
     char dt = 0;
     CK(dsx_io_read_matrix(f_img[0].c_str(), "ct_img", &rows, &cols, &dt, nullptr, 0));
     const size_t plane = (size_t)rows * cols;
-    std::vector<double> raw(plane * F), poses((size_t)rows * 6 * F);
     std::vector<std::vector<double>> granges(F);
     int n_range = 1 << 30;
-    for (int k = 0; k < F; k++) {
+    for (int k = 0; k < F; k++) {                                           // header size queries; the values come below
         int r, c;
         CK(dsx_io_read_matrix(f_img[k].c_str(), "ct_img", &r, &c, &dt, nullptr, 0));
         if (r != rows || c != cols || dt != 'd') { fprintf(stderr, "%s: frames of one shape and type CV_64F expected\n", f_img[k].c_str()); return 1; }
-        CK(dsx_io_read_matrix(f_img[k].c_str(), "ct_img", &r, &c, &dt, raw.data() + plane * k, plane * 8));
         printf("image size: %d %d\n", r, c);                                // util.cpp:94
         CK(dsx_io_read_matrix(f_pose[k].c_str(), "auv_pose", &r, &c, &dt, nullptr, 0));
         if (r != rows || c != 6 || dt != 'd') { fprintf(stderr, "%s: rows x 6 CV_64F expected\n", f_pose[k].c_str()); return 1; }
-        CK(dsx_io_read_matrix(f_pose[k].c_str(), "auv_pose", &r, &c, &dt, poses.data() + (size_t)rows * 6 * k, (size_t)rows * 6 * 8));
         int n = 0;
         CK(dsx_io_read_column(f_gr[k].c_str(), nullptr, 0, &n));
         granges[k].resize(n);
@@ -94,6 +91,17 @@ int main(int argc, char** argv) {
     // GetNormalizeSSS, GetFilteredMask, the geo look-ups and DetectFeature run inside the survey call on the raw frames
     dsx_ctx* ctx = nullptr;
     CK(dsx_create(nullptr, nullptr, &ctx));                                  // ORBextractor(2000, 1.2, 6, 12, 7), frame.cpp:180
+    // the ct_img / auv_pose values: the files' decimal text converted on the GPU.  One GPU: the raw frames stay in device
+    // memory, where dsx_survey_raw_host reads them in place; --gpus N: page-locked host memory, from which every device
+    // of the group copies its own frames
+    double* raw = nullptr;
+    if (gpus > 1) CU(cudaMallocHost((void**)&raw, sizeof(double) * plane * F));
+    else CU(cudaMalloc((void**)&raw, sizeof(double) * plane * F));
+    std::vector<const char*> p_img(F), p_pose(F);
+    for (int k = 0; k < F; k++) { p_img[k] = f_img[k].c_str(); p_pose[k] = f_pose[k].c_str(); }
+    std::vector<double> poses((size_t)rows * 6 * F);
+    CK(dsx_io_read_matrix_batch(ctx, p_img.data(), F, "ct_img", rows, cols, raw, cols, plane, nullptr));
+    CK(dsx_io_read_matrix_batch(ctx, p_pose.data(), F, "auv_pose", rows, 6, poses.data(), 6, (size_t)rows * 6, nullptr));
     std::vector<double> rowtab((size_t)rows * 6), bbox(4 * (size_t)F), gr_packed((size_t)n_range * F);
     for (int k = 0; k < F; k++) {
         CK(dsx_geo_model_build(poses.data() + (size_t)rows * 6 * k, rows, cols, granges[k].data(), (int)granges[k].size(), rowtab.data(),
@@ -128,11 +136,11 @@ int main(int argc, char** argv) {
         std::vector<int> devices(gpus);
         for (int d = 0; d < gpus; d++) devices[d] = d;
         CK(dsx_group_create(nullptr, devices.data(), gpus, &group));
-        CK(dsx_group_survey_raw_host(group, raw.data(), F, rows, cols, cols, plane, poses.data(), gr_packed.data(), n_range, img_id.data(),
+        CK(dsx_group_survey_raw_host(group, raw, F, rows, cols, cols, plane, poses.data(), gr_packed.data(), n_range, img_id.data(),
                                      pairs.data(), n_pairs, nullptr, &feats, d_cnt, d_off, d_rows6, cap_rows, &k_total, nullptr, nullptr,
                                      nullptr, nullptr));
     } else {
-        CK(dsx_survey_raw_host(ctx, raw.data(), F, rows, cols, cols, plane, poses.data(), gr_packed.data(), n_range, img_id.data(),
+        CK(dsx_survey_raw_host(ctx, raw, F, rows, cols, cols, plane, poses.data(), gr_packed.data(), n_range, img_id.data(),
                                pairs.data(), n_pairs, &feats, d_cnt, d_off, d_rows6, cap_rows, &k_total, nullptr, nullptr, nullptr, nullptr));
     }
     std::vector<double> rows6(6 * (size_t)std::max<int64_t>(k_total, 1));
@@ -156,6 +164,7 @@ int main(int argc, char** argv) {
     }
     dsx_features_free(&feats);
     cudaFree(d_cnt); cudaFree(d_off); cudaFree(d_rows6);
+    if (gpus > 1) cudaFreeHost(raw); else cudaFree(raw);
     if (group) dsx_group_destroy(group);
     dsx_destroy(ctx);
     return 0;

@@ -383,7 +383,7 @@ int dsx_group_survey_raw_host(dsx_group* g, const double* raw, int n_images, int
                               uint8_t* mask_out, double* stats_out);
 
 /* ------------------------------------------------------------------------------------------------
- * The reference's on-disk formats (SURVEY.md section 8f rank 4; host code, no device work), so that test_demo's inputs
+ * The reference's on-disk formats (SURVEY.md section 8f rank 4; host code, except the batch reader's conversion), so that test_demo's inputs
  * load without OpenCV / Boost.  Util::LoadInputData, src/util/util.cpp:85-210.
  * ---------------------------------------------------------------------------------------------- */
 
@@ -396,6 +396,20 @@ int dsx_io_read_matrix(const char* path, const char* node, int* rows, int* cols,
 int dsx_io_write_matrix(const char* path, const char* node, int rows, int cols, char dt, const void* data);
 /* Altitude / ground-range text files (util.cpp:127-179): one value per non-empty line.  out = NULL: count only. */
 int dsx_io_read_column(const char* path, double* out, int cap, int* n);
+/* dsx_io_read_matrix for n_files files at once, with the decimal text converted on the context's device.  Every file
+ * must hold the opencv-matrix node `node` as rows x cols of element type d (CV_64F: ct_img, auv_pose); file k's values
+ * land at out + k*stride, row r at + r*pitch (pitch, stride in doubles; padding is never written).  out may be device
+ * memory of the context's device, or host memory (pageable or page-locked).  Every value is bit for bit the double
+ * dsx_io_read_matrix returns for that file.  A file that dsx_io_read_matrix would reject fails with that status and
+ * message, naming the file.  host_values (optional) receives how many values were converted on the host: tokens the
+ * device cannot prove it converts exactly (more than 19 significant digits, bytes outside the plain decimal grammar,
+ * very long tokens, a rare inconclusive rounding step), and every value of a file whose text the device cannot split
+ * the way dsx_io_read_matrix reads it.
+ * Host threads read the files into page-locked staging slots (kept in the context, four slots of the largest file's
+ * size) while the previous files' text is copied and parsed on the device.  Synchronous: returns when every value is
+ * in out. */
+int dsx_io_read_matrix_batch(dsx_ctx* ctx, const char* const* paths, int n_files, const char* node, int rows, int cols,
+                             double* out, size_t pitch, size_t stride, int64_t* host_values);
 
 /* Synchronises the context's stream and returns DSX_ERR_CAPACITY if any kernel since the last check overflowed a
  * fixed-capacity list or the caller's rows6 buffer (the device-side error word), DSX_OK otherwise. */
