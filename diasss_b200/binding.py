@@ -52,6 +52,8 @@ EXPORTS = [
     "dsx_features_free", "dsx_detect_feature_batch_dev", "dsx_detect_feature_batch", "dsx_geo_model_build", "dsx_geo_model_build_batch", "dsx_georef_batch_dev",
     "dsx_match_pairs_dev", "dsx_survey", "dsx_frame_prepare_batch_dev", "dsx_compute_intersection", "dsx_build_pair_list", "dsx_check_error", "dsx_launch_count", "dsx_timing_enable", "dsx_timing_read", "dsx_stage_name", "dsx_popc_peak",
     "dsx_peer_create", "dsx_peer_connect", "dsx_peer_connect_local", "dsx_match_pairs_peer", "dsx_peer_collect", "dsx_peer_destroy",
+    "dsx_ranks_create", "dsx_ranks_connect", "dsx_ranks_connect_local", "dsx_ranks_publish_host", "dsx_ranks_publish_raw_host",
+    "dsx_ranks_match", "dsx_ranks_destroy",
     "dsx_group_create", "dsx_group_destroy", "dsx_group_ctx", "dsx_group_blocks", "dsx_group_survey_host", "dsx_group_survey_raw_host",
     "dsx_io_read_matrix", "dsx_io_write_matrix", "dsx_io_read_column", "dsx_io_read_matrix_batch",
     "dsx_debug_level_image", "dsx_debug_candidates", "dsx_debug_level_keys", "dsx_debug_match", "dsx_debug_sincosf", "dsx_debug_fast_profile", "dsx_survey_host", "dsx_survey_raw_host", "dsx_get_kps_pairs_dev",
@@ -77,6 +79,7 @@ def lib():
         L.dsx_default_params.restype = None
         L.dsx_peer_destroy.restype = None
         L.dsx_group_destroy.restype = None
+        L.dsx_ranks_destroy.restype = None
         L.dsx_group_ctx.restype = C.c_void_p
         _lib = L
     return _lib
@@ -408,6 +411,68 @@ class Peer:
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
             lib().dsx_peer_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class Ranks:
+    """dsx_ranks: this rank's end of a survey run with one process per GPU (see include/diasss_b200.h).  Per step call
+    publish_host / publish_raw_host (this rank's frames only), then match (all frames' ids and boxes, the whole pair list)."""
+    HANDLE_BYTES = 64
+
+    def __init__(self, ctx, rank, world, n_images, n_pairs, cap_rows, image_counts=None):
+        self.ctx, self.rank, self.world, self.n_images, self.n_pairs, self.cap_rows = ctx, rank, world, n_images, n_pairs, cap_rows
+        counts = None if image_counts is None else np.ascontiguousarray(image_counts, np.int32)
+        if counts is not None and len(counts) != world:
+            raise DsxError(ERR_INVALID, "image_counts needs one entry per rank")
+        self.first = group_blocks(n_images, world, counts)
+        self.count = int(self.first[rank + 1] - self.first[rank])
+        self._h = C.c_void_p()
+        self.handle = np.zeros(self.HANDLE_BYTES, np.uint8)
+        _chk(lib().dsx_ranks_create(ctx._h, int(rank), int(world), int(n_images), _p(counts), int(n_pairs), C.c_int64(cap_rows),
+                                    C.byref(self._h), _p(self.handle)))
+
+    def connect(self, handles):
+        handles = np.ascontiguousarray(handles, np.uint8).reshape(self.world, self.HANDLE_BYTES)
+        _chk(lib().dsx_ranks_connect(self._h, _p(handles)))
+
+    def connect_local(self, q, other):
+        _chk(lib().dsx_ranks_connect_local(self._h, int(q), other._h))
+
+    def publish_host(self, images_ptr, masks_ptr, rows, cols, step, img_stride, poses, g_ranges, bbox_out=None):
+        """Phase 1: this rank's frames (images / masks, poses [count, rows, 6], g_ranges [count, n_range])."""
+        assert poses.dtype == np.float64 and poses.flags.c_contiguous and g_ranges.dtype == np.float64 and g_ranges.flags.c_contiguous
+        _chk(lib().dsx_ranks_publish_host(self._h, _p(images_ptr), _p(masks_ptr) if masks_ptr else C.c_void_p(0), rows, cols,
+                                          C.c_size_t(step), C.c_size_t(img_stride), _p(poses), _p(g_ranges), g_ranges.shape[-1],
+                                          _p(bbox_out)))
+
+    def publish_raw_host(self, raw_ptr, rows, cols, raw_pitch, raw_stride, poses, g_ranges, bbox_out=None, norm_out=None,
+                         mask_out=None, stats_out=None):
+        """Phase 1 from raw float64 frames of this rank (pitch and stride in doubles)."""
+        assert poses.dtype == np.float64 and poses.flags.c_contiguous and g_ranges.dtype == np.float64 and g_ranges.flags.c_contiguous
+        _chk(lib().dsx_ranks_publish_raw_host(self._h, _p(raw_ptr), rows, cols, C.c_size_t(raw_pitch), C.c_size_t(raw_stride), _p(poses),
+                                              _p(g_ranges), g_ranges.shape[-1], _p(bbox_out), _p(norm_out), _p(mask_out), _p(stats_out)))
+
+    def match(self, img_id, bbox, pairs, feats=None, corr_count_ptr=None, corr_offset_ptr=None, rows6_ptr=None, sync=True):
+        """Phase 2.  Rank 0 passes its output buffers; returns the row total (rank 0) or this rank's rows when sync."""
+        img_id = np.ascontiguousarray(img_id, np.int32)
+        bbox = np.ascontiguousarray(bbox, np.float64)
+        pairs = np.ascontiguousarray(pairs, np.int32).reshape(-1, 2)
+        if len(pairs) != self.n_pairs:
+            raise DsxError(ERR_INVALID, "pairs: the object was created for %d pairs" % self.n_pairs)
+        kt = C.c_int64()
+        _chk(lib().dsx_ranks_match(self._h, _p(img_id), _p(bbox), _p(pairs), C.byref(feats) if feats is not None else C.c_void_p(0),
+                                   _p(corr_count_ptr), _p(corr_offset_ptr), _p(rows6_ptr), C.byref(kt) if sync else C.c_void_p(0)))
+        return kt.value if sync else None
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h.value:
+            lib().dsx_ranks_destroy(self._h)
             self._h = C.c_void_p()
 
     def __del__(self):

@@ -284,6 +284,9 @@ int match_pairs(dsx_ctx* ctx, const dsx_features_dev* feats, const int32_t* img_
 int match_begin(dsx_ctx* ctx, const dsx_features_dev* feats, const int32_t* img_id, const int32_t* img_rows, const double* bbox,
                 const int32_t* pairs, const int32_t* slot_of, int n_pairs, int32_t* dbg_corres, int32_t* dbg_scc_count, double* dbg_scc_model);
 int match_stage(dsx_ctx* ctx, const dsx_features_dev* feats, int img_first, int img_count, int pair_first, int pair_count);
+// grows the matcher scratch to what match_begin needs for (cap, nimg, n_pairs) without a slot map, ahead of the call (the
+// growth synchronises the stream and frees device memory, which must not happen behind a kernel spinning on a peer)
+int match_reserve(dsx_ctx* ctx, int cap, int nimg, int n_pairs);
 int match_finish(dsx_ctx* ctx, const dsx_features_dev* feats, int32_t* corr_count, int32_t* corr_offset, double* rows6, int64_t cap_rows,
                  int64_t* k_total, int32_t* dbg_idx);
 int match_finish_peer(dsx_ctx* ctx, const dsx_features_dev* feats, int32_t* l_cnt, int32_t* l_off, const PeerPub& pub, const PeerSink& sink,

@@ -1084,11 +1084,9 @@ static int ensure_scratch(dsx_ctx* ctx, size_t bytes) {
 //   match_stage   sorts the keypoints of images [img_first, img_first+img_count) along the search axis and runs K7 + K8/K9
 //                 for slots [pair_first, pair_first+pair_count) (whose images must all be prepared by then).
 //   match_finish  scans the counts in output order and emits the rows.
-int match_begin(dsx_ctx* ctx, const dsx_features_dev* feats, const int32_t* img_id, const int32_t* img_rows, const double* bbox,
-                const int32_t* pairs, const int32_t* slot_of, int n_pairs, int32_t* dbg_corres, int32_t* dbg_scc_count, double* dbg_scc_model) {
+static size_t match_layout(dsx_ctx* ctx, int cap, int nimg, int n_pairs, bool has_slots) {
     MatchPlan& M = ctx->mplan;
-    const int cap = feats->cap, nimg = feats->n_images;
-    M.cap = cap; M.nimg = nimg; M.n_pairs = n_pairs; M.has_slots = slot_of != nullptr;
+    M.cap = cap; M.nimg = nimg; M.n_pairs = n_pairs; M.has_slots = has_slots;
     M.big = (size_t)cap * 16 > 160 * 1024;      // per-keypoint working arrays of K7/K8 move to global scratch
     {   // K7 form: warp-autonomous for dense images (DSX_MATCH_AUTON: 1 always, 0 never); its per-target state moves to
         // global scratch when it does not fit next to the warps' staging slices
@@ -1116,8 +1114,18 @@ int match_begin(dsx_ctx* ctx, const dsx_features_dev* feats, const int32_t* img_
     if (cap > kSortMax) { M.g_n2 = 1; while (M.g_n2 < cap) M.g_n2 <<= 1; }
     M.o_gv = M.o_gk + sizeof(unsigned long long) * (size_t)nimg * M.g_n2;
     M.o_col = (M.o_gv + sizeof(int) * (size_t)nimg * M.g_n2 + 15) & ~(size_t)15;
-    const size_t total = M.o_col + sizeof(int32_t) * (size_t)nimg * (kMaxCol + 1);
-    DSX_TRY(ensure_scratch(ctx, total));
+    return M.o_col + sizeof(int32_t) * (size_t)nimg * (kMaxCol + 1);
+}
+
+int match_reserve(dsx_ctx* ctx, int cap, int nimg, int n_pairs) {
+    return ensure_scratch(ctx, match_layout(ctx, cap, nimg, n_pairs, false));
+}
+
+int match_begin(dsx_ctx* ctx, const dsx_features_dev* feats, const int32_t* img_id, const int32_t* img_rows, const double* bbox,
+                const int32_t* pairs, const int32_t* slot_of, int n_pairs, int32_t* dbg_corres, int32_t* dbg_scc_count, double* dbg_scc_model) {
+    MatchPlan& M = ctx->mplan;
+    const int cap = feats->cap, nimg = feats->n_images;
+    DSX_TRY(ensure_scratch(ctx, match_layout(ctx, cap, nimg, n_pairs, slot_of != nullptr)));
     uint8_t* S = (uint8_t*)ctx->m_scratch;
     DSX_CUDA(cudaMemcpyAsync(S + M.o_id, img_id, sizeof(int32_t) * nimg, cudaMemcpyHostToDevice, ctx->stream));
     DSX_CUDA(cudaMemcpyAsync(S + M.o_rows, img_rows, sizeof(int32_t) * nimg, cudaMemcpyHostToDevice, ctx->stream));

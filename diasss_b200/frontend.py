@@ -181,13 +181,17 @@ class FrontEnd:
                                      out["offset"].data_ptr(), out["rows6"].data_ptr(), out["rows6"].shape[0], sync=sync)
         return dict(feats=feats, count=out["count"], offset=out["offset"], rows6=out["rows6"][:k] if sync else out["rows6"], k=k)
 
+    def rows_per_pair(self, n_pairs):
+        """The row reservation per pair alloc_match_out makes by default."""
+        return 2 * self.ctx.cap if max(n_pairs, 1) * 2 * self.ctx.cap * 48 <= (1 << 30) else 1024
+
     def alloc_match_out(self, n_pairs, dev, rows_per_pair=None):
         """Output block of the pair matcher.  A pair can emit at most 2*cap rows (every keypoint of both frames);
         that worst case is reserved while it stays under 1 GB, otherwise 1024 rows per pair (DSX_ERR_CAPACITY if
         a survey ever exceeds it)."""
         import torch
         if rows_per_pair is None:
-            rows_per_pair = 2 * self.ctx.cap if max(n_pairs, 1) * 2 * self.ctx.cap * 48 <= (1 << 30) else 1024
+            rows_per_pair = self.rows_per_pair(n_pairs)
         return dict(count=torch.zeros(max(n_pairs, 1), dtype=torch.int32, device=dev),
                     offset=torch.zeros(n_pairs + 1, dtype=torch.int32, device=dev),
                     rows6=torch.zeros(max(n_pairs, 1) * rows_per_pair, 6, dtype=torch.float64, device=dev))

@@ -209,3 +209,116 @@ class PeerCollector:
         if self.peer is not None:
             self.peer.close()
             self.peer = None
+
+
+def directory_exchange(directory, rank, world, handle, timeout_s=120.0):
+    """Exchanges the ranks' 64-byte handles through a shared directory: rank r writes DIR/handle.<r> by rename (so a reader
+    never sees a partial file) and polls for the others.  Returns [world, 64] uint8, rank-major."""
+    import os
+    import time
+    handle = np.ascontiguousarray(handle, np.uint8).reshape(-1)
+    tmp = os.path.join(directory, "handle.%d.tmp" % rank)
+    with open(tmp, "wb") as f:
+        f.write(handle.tobytes())
+    os.replace(tmp, os.path.join(directory, "handle.%d" % rank))
+    out = np.zeros((world, handle.size), np.uint8)
+    t0 = time.monotonic()
+    for q in range(world):
+        path = os.path.join(directory, "handle.%d" % q)
+        while not os.path.exists(path):
+            if time.monotonic() - t0 > timeout_s:
+                raise TimeoutError("no handle from rank %d in %s" % (q, directory))
+            time.sleep(0.01)
+        out[q] = np.frombuffer(open(path, "rb").read(), np.uint8)
+    return out
+
+
+def _dist_exchange(rank, world, handle):
+    got = [None] * world
+    dist.all_gather_object(got, bytes(np.ascontiguousarray(handle, np.uint8).tobytes()))
+    return np.stack([np.frombuffer(g, np.uint8) for g in got])
+
+
+class RankSurvey:
+    """One rank of a survey run with one process per GPU through the library alone (dsx_ranks_* in
+    include/diasss_b200.h): no NCCL and no host collective per step.
+
+    publish() / publish_raw()  phase 1: this rank's frames (self.first[rank] .. self.first[rank + 1]) are extracted and
+                               their features published to every rank.  Returns this rank's boxes [count, 4].
+    match()                    phase 2: every frame's ids and boxes and the whole pair list; rank 0 returns
+                               dict(feats, count, offset, rows6, k) exactly as FrontEnd.process_survey_host for the whole
+                               survey, another rank dict(k=rows it matched).
+    The handles are exchanged once, at set-up: through torch.distributed (all_gather_object) by default, or by
+    `exchange(handle) -> [world, 64] uint8` (directory_exchange, say); exchange=False leaves the connection to the caller
+    (connect_local for ranks of one process).  n_pairs and the output capacity are fixed for the object's life.  Close a
+    rank only once rank 0's last step has completed: until then the other ranks' kernels may still store into its memory."""
+
+    def __init__(self, frontend, rank, world, n_images, n_pairs, rows_per_pair=None, image_counts=None, exchange=None, cap_rows=None):
+        """cap_rows: rows rank 0 can hold (default n_pairs x rows_per_pair, by default FrontEnd.alloc_match_out's reservation)."""
+        from . import binding as B
+        self.fe, self.rank, self.world, self.n_images, self.n_pairs = frontend, int(rank), int(world), int(n_images), int(n_pairs)
+        self.dev = torch.device("cuda", frontend.ctx.params.device if frontend.ctx.params.device >= 0 else torch.cuda.current_device())
+        # every rank is created with the same row capacity; only rank 0 holds output buffers
+        if cap_rows is None:
+            cap_rows = max(self.n_pairs, 1) * int(rows_per_pair or frontend.rows_per_pair(self.n_pairs))
+        self.cap_rows = int(cap_rows)
+        self.out = self.feats = None
+        if self.rank == 0:
+            with torch.cuda.device(self.dev):
+                self.out = dict(count=torch.zeros(max(self.n_pairs, 1), dtype=torch.int32, device=self.dev),
+                                offset=torch.zeros(self.n_pairs + 1, dtype=torch.int32, device=self.dev),
+                                rows6=torch.zeros(self.cap_rows, 6, dtype=torch.float64, device=self.dev))
+                self.feats = frontend.alloc_features(self.n_images)
+                torch.cuda.synchronize(self.dev)    # (the zeroed buffers are written on the context's stream)
+        self.ranks = B.Ranks(frontend.ctx, self.rank, self.world, self.n_images, self.n_pairs, self.cap_rows, image_counts)
+        self.first = self.ranks.first
+        self.count = self.ranks.count
+        if exchange is not False:
+            handles = (exchange or (lambda h: _dist_exchange(self.rank, self.world, h)))(self.ranks.handle)
+            self.ranks.connect(handles)
+
+    def connect_local(self, others):
+        """Same-process ranks: `others` = every rank's RankSurvey (this one included)."""
+        for q, o in enumerate(others):
+            if q != self.rank:
+                self.ranks.connect_local(q, o.ranks)
+
+    def publish(self, images, masks, poses, g_ranges):
+        from .frontend import _host_ptr
+        n, rows, cols = self._shape(images)
+        poses = np.ascontiguousarray(poses, np.float64).reshape(n, rows, 6)
+        g_ranges = np.ascontiguousarray(g_ranges, np.float64).reshape(n, np.shape(g_ranges)[-1])
+        bbox = np.zeros((n, 4), np.float64)
+        self.rows = rows
+        self.ranks.publish_host(_host_ptr(images), _host_ptr(masks), rows, cols, cols, rows * cols, poses, g_ranges, bbox)
+        return bbox
+
+    def publish_raw(self, raws, poses, g_ranges, prepared=False):
+        """publish() from raw float64 frames (host or this GPU); prepared=True also returns norm / mask / stats."""
+        from .frontend import _raw_view
+        n, rows, cols = self._shape(raws)
+        ptr, pitch, stride = _raw_view(raws)
+        poses = np.ascontiguousarray(poses, np.float64).reshape(n, rows, 6)
+        g_ranges = np.ascontiguousarray(g_ranges, np.float64).reshape(n, np.shape(g_ranges)[-1])
+        bbox = np.zeros((n, 4), np.float64)
+        host = {}
+        if prepared:
+            host = dict(norm=np.zeros((n, rows, cols), np.uint8), mask=np.zeros((n, rows, cols), np.uint8), stats=np.zeros((n, 3), np.float64))
+        self.ranks.publish_raw_host(ptr, rows, cols, pitch, stride, poses, g_ranges, bbox, host.get("norm"), host.get("mask"), host.get("stats"))
+        return (bbox, host) if prepared else bbox
+
+    def match(self, img_ids, bboxes, pairs, sync=True):
+        o = self.out
+        if self.rank != 0:
+            return dict(k=self.ranks.match(img_ids, bboxes, pairs, sync=sync))
+        k = self.ranks.match(img_ids, bboxes, pairs, self.feats["c"], o["count"].data_ptr(), o["offset"].data_ptr(),
+                             o["rows6"].data_ptr(), sync=sync)
+        return dict(feats=self.feats, count=o["count"], offset=o["offset"], rows6=o["rows6"][:k] if sync else o["rows6"], k=k)
+
+    def _shape(self, a):
+        if a.shape[0] != self.count:
+            raise ValueError("rank %d publishes %d frames, got %d" % (self.rank, self.count, a.shape[0]))
+        return tuple(int(s) for s in a.shape)
+
+    def close(self):
+        self.ranks.close()

@@ -341,6 +341,59 @@ int dsx_peer_collect(dsx_ctx* ctx, dsx_peer* peer, int seq, const int32_t** corr
 void dsx_peer_destroy(dsx_peer* peer);
 
 /* ------------------------------------------------------------------------------------------------
+ * One process per GPU through this library alone (no NCCL, no host collective per step).  Rank r extracts its own
+ * contiguous block of frames (dealt as dsx_group_blocks deals them, so the gathered feature block is in image order),
+ * publishes the counted rows of their features into every rank's memory over peer links, matches the r-th contiguous
+ * block of the pair list and writes its rows into rank 0's memory behind the lower ranks' rows (dsx_match_pairs_peer).
+ * Rank 0's outputs are byte for byte what dsx_survey_host (dsx_survey_raw_host) on one context returns for the whole
+ * survey.  The only host exchange is the ranks' 64-byte handles, once.
+ *   dsx_ranks_create   this rank's object: one device allocation (flags, both halves of the gathered feature block, the
+ *                      row collection; rank 0's also 2 x cap_rows rows), exported as one CUDA IPC handle.  Every rank
+ *                      passes the same world, n_images, image_counts (NULL = equal split), n_pairs and cap_rows, which
+ *                      stay fixed for the object's life, and a context with the same parameters.  The matcher scratch
+ *                      of every later step is sized here.
+ *   dsx_ranks_connect  maps the other ranks' allocations; handles = world x DSX_IPC_HANDLE_BYTES bytes, rank-major.
+ *   dsx_ranks_connect_local  same-process ranks: rank q's allocation is `other`'s (no IPC).
+ *   phase 1  dsx_ranks_publish_host / dsx_ranks_publish_raw_host  extract THIS rank's frames (images / raw, pose6,
+ *            g_range, bbox_out and the optional planes hold this rank's count_r frames only; arguments as for
+ *            dsx_survey_host / dsx_survey_raw_host) and publish their features to every rank.  Never waits for a peer.
+ *            bbox_out (count_r x 4, may be NULL) is complete on return.
+ *   phase 2  dsx_ranks_match  waits ON THE DEVICE until every rank has published this step, matches this rank's block of
+ *            the pair list (n_pairs pairs of indices into all frames), rows to rank 0.  img_id (n_images) and bbox
+ *            (n_images x 4, dsx_geo_model_build_batch of every frame's poses) cover ALL frames; this rank's own boxes
+ *            must equal the ones phase 1 computed, else DSX_ERR_INVALID and nothing is enqueued.  On rank 0, feats (a
+ *            block from dsx_features_alloc with room for n_images; only the bytes of counted rows are written), corr_count,
+ *            corr_offset and rows6 (device, 16-byte aligned, as dsx_survey_host) receive the outputs; elsewhere they may
+ *            be NULL.  k_total non-NULL: the call synchronises; rank 0 stores the row total and reports
+ *            DSX_ERR_CAPACITY when the ranks' rows exceed cap_rows, DSX_ERR_CUDA when another rank failed the step or a
+ *            wait timed out; another rank stores the rows it matched and reports its own errors.  k_total NULL: enqueue
+ *            only; on rank 0 the whole cap_rows rows of rows6 are copied and dsx_check_error reports a failed step.
+ * Each step is one publish followed by one match on every rank; an argument error leaves the step where it was.
+ * Why two phases: a rank's wait depends on every rank (the row collection's waits only on lower ranks), and the library
+ * synchronises a whole device when it grows staging.  A process that drives several ranks must therefore enqueue the
+ * publish of EVERY rank before any match, then the matches (with k_total NULL, except on the last one called); a caller
+ * with one process per GPU simply calls the two phases in sequence.  Errors stay in a rank's context until read
+ * (k_total or dsx_check_error): a rank whose error is unread forwards it to rank 0 again at the next step.
+ * The halves of the exchange are double-buffered on the step's parity and need no back-pressure: a rank publishes step
+ * s + 2 only after its wait for step s + 1, which every rank passes only after finishing its reads of step s.  A wait
+ * gives up after DSX_PEER_TIMEOUT_MS milliseconds (default 20000).  Destroy a rank only once rank 0's last step has
+ * completed (its synchronised dsx_ranks_match): until then the other ranks' kernels may still store into its allocation.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct dsx_ranks dsx_ranks;
+int dsx_ranks_create(dsx_ctx* ctx, int rank, int world, int n_images, const int32_t* image_counts, int n_pairs, int64_t cap_rows,
+                     dsx_ranks** out, uint8_t* handle);
+int dsx_ranks_connect(dsx_ranks* x, const uint8_t* handles);
+int dsx_ranks_connect_local(dsx_ranks* x, int q, dsx_ranks* other);
+int dsx_ranks_publish_host(dsx_ranks* x, const uint8_t* images, const uint8_t* masks, int rows, int cols, size_t step, size_t img_stride,
+                           const double* pose6, const double* g_range, int n_range, double* bbox_out);
+int dsx_ranks_publish_raw_host(dsx_ranks* x, const double* raw, int rows, int cols, size_t raw_pitch, size_t raw_stride,
+                               const double* pose6, const double* g_range, int n_range, double* bbox_out, uint8_t* norm_out,
+                               uint8_t* mask_out, double* stats_out);
+int dsx_ranks_match(dsx_ranks* x, const int32_t* img_id, const double* bbox, const int32_t* pairs, dsx_features_dev* feats,
+                    int32_t* corr_count, int32_t* corr_offset, double* rows6, int64_t* k_total);
+void dsx_ranks_destroy(dsx_ranks* x);
+
+/* ------------------------------------------------------------------------------------------------
  * Several GPUs from one process (SURVEY.md section 5: single process, n devices, plain peer copies; no MPI, NCCL or IPC
  * handles).  A group holds one dsx_ctx per entry of devices[], each with its own stream and host worker thread.  A device
  * may be listed more than once (logical ranks on one GPU, as dsx_peer_connect_local allows).
