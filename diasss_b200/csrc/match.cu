@@ -72,6 +72,19 @@ __device__ __forceinline__ double dkey_inv(unsigned long long k) {
     return __longlong_as_double((long long)b);
 }
 
+// Keys bounding the sort-axis window of a group of sources whose coordinates span [amin, amax].  A NaN sorts first
+// (sign bit set) or last, so a group that holds one has a NaN for amin or amax; arithmetic on a NaN gives a NaN whose
+// key lands anywhere in the order (between the negative and the positive coordinates on sm_100), which would cut real
+// coordinates out of the window.  A NaN bound opens the window on its side instead.
+__device__ __forceinline__ unsigned long long window_lo(double amin, double reach) {
+    const double v = amin - reach - fabs(amin) * 1e-15;
+    return (amin == amin && v == v) ? dkey(v) : 0ull;
+}
+__device__ __forceinline__ unsigned long long window_hi(double amax, double reach) {
+    const double v = amax + reach + fabs(amax) * 1e-15;
+    return (amax == amax && v == v) ? dkey(v) : ~0ull;
+}
+
 // column of the other-axis coordinate o (clamped; NaN -> 0).  |o1 - o2| < col_w  =>  the columns differ by at most one.
 __device__ __forceinline__ int col_of(double o, double org, double w, int ncol) {
     const double t = floor((o - org) / w);
@@ -285,8 +298,8 @@ __global__ void __launch_bounds__(kMatchThreads, 1) match_pair_kernel(const Pair
         bool warp_active = p0 < ns;
         if (CULL && warp_active) {
             const double amin = dkey_inv(skey_a[p0]), amax = dkey_inv(skey_a[min(p0 + 32 * SPT, ns) - 1]);
-            klo = dkey(amin - A.reach - fabs(amin) * 1e-15);
-            khi = dkey(amax + A.reach + fabs(amax) * 1e-15);
+            klo = window_lo(amin, A.reach);
+            khi = window_hi(amax, A.reach);
             double omn = INFINITY, omx = -INFINITY;
 #pragma unroll
             for (int s = 0; s < SPT; s++)
@@ -306,7 +319,7 @@ __global__ void __launch_bounds__(kMatchThreads, 1) match_pair_kernel(const Pair
             const unsigned long long ka0 = skey_a[sb], ka1 = skey_a[min(sb + kMatchThreads * SPT, ns) - 1];
             if (!(ka0 == 0ull && ka1 == 0ull)) {
                 const double bmin = dkey_inv(ka0), bmax = dkey_inv(ka1);
-                const unsigned long long blo = dkey(bmin - A.reach - fabs(bmin) * 1e-15), bhi = dkey(bmax + A.reach + fabs(bmax) * 1e-15);
+                const unsigned long long blo = window_lo(bmin, A.reach), bhi = window_hi(bmax, A.reach);
                 int lo = 0, hi = nt;
                 while (lo < hi) { const int mid = (lo + hi) >> 1; if (skey_b[mid] < blo) lo = mid + 1; else hi = mid; }
                 jlo = lo; hi = nt;
@@ -603,7 +616,7 @@ __global__ void __launch_bounds__(kMatchThreads, 1) match_pair_auton_kernel(cons
         const bool windowed = tgt_sorted && !(ka0 == 0ull && ka1 == 0ull);
         // the group's interval on the sort axis (decoded conservatively from the truncated composite keys)
         const double amin = dkey_inv(comp ? (ka0 & m56) << 8 : ka0), amax = dkey_inv(comp ? ((ka1 & m56) << 8) | 0xffull : ka1);
-        const unsigned long long wlo = dkey(amin - A.reach - fabs(amin) * 1e-15), whi = dkey(amax + A.reach + fabs(amax) * 1e-15);
+        const unsigned long long wlo = window_lo(amin, A.reach), whi = window_hi(amax, A.reach);
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) { omn = fmin(omn, __shfl_xor_sync(0xffffffffu, omn, o)); omx = fmax(omx, __shfl_xor_sync(0xffffffffu, omx, o)); }
         const double org_o = A.axis ? A.org_x : A.org_y;
